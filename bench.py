@@ -16,6 +16,11 @@ the sorted monitored draws for the rank normalisation, all-reduce of the ESS / R
 inside the timed `e2e_with_diagnostics` number.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c5|c3|c2|c3small|c2small]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed engine call returned (positions, momenta, energies, gradients, acceptance
+statistics, tree depths, flags, leapfrog counts, counters) as DIR/<name>.npy, so that two builds run with the same arguments
+-- hence the same seeded inputs -- can be compared output for output (see last_step_outputs).
 """
 import argparse
 import json
@@ -43,6 +48,8 @@ EPS = {"dense": 0.25, "logistic": 0.4}
 METRIC = "leapfrog_gradient_evals_per_sec"
 UNIT = "gradient evals/s"
 MIN_TIMED_S = 2.0          # secondary workloads choose their step count so that the timed region lasts this long
+DUMP_BYTES = 64 * 10 ** 6  # --dump-outputs: all files together stay within this
+DUMP_ROW_BYTES = 48 << 20  # ... of which the three [chains, dim] arrays take at most this (a seeded sample of the chains)
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -466,7 +473,48 @@ def build_problem(name, dev):
     return model, metric, dtype, dtype_name
 
 
-def run_tick_workload(name, D, steps, warmup, min_timed_s=0.0, with_e2e=True):
+def dump_rows(Cn, d, esize):
+    """Chains whose [dim] rows --dump-outputs writes: all of them when the three [chains, dim] arrays fit DUMP_ROW_BYTES,
+    else a fixed, seeded sample in ascending order (the same chains in every run)."""
+    n = min(Cn, DUMP_ROW_BYTES // (3 * d * esize))
+    if n == Cn:
+        return np.arange(Cn)
+    return np.sort(np.random.default_rng(0).choice(Cn, n, replace=False))
+
+
+def _host_float(t):
+    a = t.detach().cpu().numpy()
+    return a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)     # int / bool: exact in float64
+
+
+def last_step_outputs(info, extras, rows, chain_offset=0):
+    """Host copies of what one engine call returned to its caller: the [chains, dim] arrays at `rows` only, every
+    per-chain array in full, the call's counters (leapfrogs, transitions, ticks, chain-ticks) and the global ids of
+    `rows` as `chains`.  Float arrays keep their dtype; integer and boolean arrays become float64."""
+    import torch
+    st = info.state
+    idx = torch.from_numpy(np.asarray(rows, dtype=np.int64)).to(st.position.device)
+    out = {"chains": (chain_offset + np.asarray(rows)).astype(np.float64)}
+    for k in ("position", "momentum", "potential_energy_grad"):
+        out[k] = _host_float(getattr(st, k).index_select(0, idx))
+    out["potential_energy"] = _host_float(st.potential_energy)
+    for k in ("acceptance_probability", "num_doublings", "is_turning", "is_diverging"):
+        out[k] = _host_float(getattr(info, k))
+    out["n_leapfrog"] = _host_float(extras["n_leapfrog"])
+    out["counters"] = _host_float(extras["counters"])
+    return out
+
+
+def write_outputs(path, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise ValueError(f"outputs of {total} bytes exceed the {DUMP_BYTES}-byte limit of --dump-outputs")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
+def run_tick_workload(name, D, steps, warmup, min_timed_s=0.0, with_e2e=True, dump=False):
     """Device-resident and end-to-end throughput of one tick-engine workload.  Returns a dict (rank-reduced)."""
     import torch
     import aehmc_b200 as ab
@@ -494,7 +542,7 @@ def run_tick_workload(name, D, steps, warmup, min_timed_s=0.0, with_e2e=True):
         info, ex = _engine.run("nuts", model, metric, srng, state, eps, max_ticks=ticks, resume=True,
                                workspace_key=key, return_counters=True)
         state = info.state
-        last["info"] = info
+        last["info"], last["extras"] = info, ex
         return ex["counters"]
 
     warm = max(warmup, 3)
@@ -516,6 +564,8 @@ def run_tick_workload(name, D, steps, warmup, min_timed_s=0.0, with_e2e=True):
     D.barrier()
     ms_total = ev0.elapsed_time(ev1)
     clocks = sampler.stop()
+    # every engine call returns fresh tensors: these are the last timed call's, copied out before the extra calls below
+    outputs = last_step_outputs(last["info"], last["extras"], dump_rows(Cn, d, esize), chain_offset) if dump else None
     cnt = torch.stack(counters).sum(0).cpu().numpy()      # leapfrogs, transitions, ticks(unused), chain-ticks
     acc = last["info"].acceptance_probability
     ms_total = D.reduce([ms_total], "max")[0]
@@ -526,7 +576,8 @@ def run_tick_workload(name, D, steps, warmup, min_timed_s=0.0, with_e2e=True):
            "dtype": dtype, "dtype_name": dtype_name, "clocks": clocks, "model": model, "metric": metric,
            "transitions_per_step": total_transitions / steps,
            "mean_leapfrogs_per_transition": total_leapfrogs / max(total_transitions, 1.0),
-           "mean_accept": acc_sum / (Cn * D.world), "esize": esize, "q_host": q_host, "chain_offset": chain_offset}
+           "mean_accept": acc_sum / (Cn * D.world), "esize": esize, "q_host": q_host, "chain_offset": chain_offset,
+           "outputs": outputs}
 
     # ---- the tick kernel (integrator + U-turn + proposal bookkeeping of one leapfrog of every chain) timed on its own:
     #      b2h_tick_timer brackets each of its launches with CUDA events on the engine's stream (outside the headline
@@ -803,7 +854,9 @@ def run_gpu_arm(args):
     D = Dist()
     peaks = load_peaks()
     name = args.workload
-    w = run_tick_workload(name, D, args.steps, args.warmup)
+    w = run_tick_workload(name, D, args.steps, args.warmup, dump=args.dump_outputs is not None)
+    if args.dump_outputs is not None and D.rank == 0:
+        write_outputs(args.dump_outputs, w.pop("outputs"))
     roofline, roofline_elementwise = rooflines_for(w, D, peaks)
     kind, Cn, d, ticks = w["kind"], w["chains_per_gpu"], w["dim"], w["ticks"]
     kernels_per_tick = 6 if kind == "dense" else 4
@@ -879,7 +932,13 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary workloads (c3, c2, c4, c1)")
     ap.add_argument("--ess-transitions", type=int, default=200, help="kept NUTS transitions of the ESS leg")
     ap.add_argument("--ess-warmup", type=int, default=100, help="pooled window-adaptation transitions before them")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (rank 0's chains; at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -35,6 +35,40 @@ def test_reference_arm_sample_is_bounded():
     assert "configs[1]" in bench.describe("c2") and "configs[2]" in bench.describe("c3") and "configs[4]" in bench.describe("c5")
 
 
+@pytest.mark.parametrize("name", ["c5", "c2", "c3small"])
+def test_dump_outputs_fixed_sample_float_files_within_64_mb(tmp_path, name):
+    """--dump-outputs at the workload's own shape: the same seeded chain sample every time, every file float32 / float64
+    and equal to what the engine call returned (integers and flags exactly), all files together within 64 MB."""
+    torch = pytest.importorskip("torch")
+    from types import SimpleNamespace as NS
+    kind, Cn, d, _, _ = bench.WORKLOADS[name]
+    dt = torch.float64 if kind == "dense" else torch.float32
+    esize = 8 if kind == "dense" else 4
+    rows = bench.dump_rows(Cn, d, esize)
+    assert np.array_equal(rows, bench.dump_rows(Cn, d, esize)) and np.all(np.diff(rows) > 0) and rows[-1] < Cn
+    g = torch.Generator().manual_seed(0)
+    st = NS(position=torch.randn((Cn, d), generator=g, dtype=dt), momentum=torch.randn((Cn, d), generator=g, dtype=dt),
+            potential_energy=torch.randn(Cn, generator=g, dtype=dt),
+            potential_energy_grad=torch.randn((Cn, d), generator=g, dtype=dt))
+    info = NS(state=st, acceptance_probability=torch.rand(Cn, generator=g, dtype=torch.float64),
+              num_doublings=torch.randint(0, 11, (Cn,), generator=g, dtype=torch.int32),
+              is_turning=torch.rand(Cn, generator=g) < 0.5, is_diverging=torch.rand(Cn, generator=g) < 0.1)
+    extras = {"n_leapfrog": torch.randint(1, 1024, (Cn,), generator=g, dtype=torch.int32),
+              "counters": torch.tensor([123456789012, 4096, 32, Cn * 32], dtype=torch.int64)}
+    out = bench.last_step_outputs(info, extras, rows, chain_offset=Cn)
+    bench.write_outputs(str(tmp_path), out)
+    files = {p.stem: np.load(p) for p in tmp_path.glob("*.npy")}
+    assert set(files) == set(out) and sum(a.nbytes for a in files.values()) <= bench.DUMP_BYTES <= 64 * 10 ** 6
+    assert all(a.dtype in (np.float32, np.float64) for a in files.values())
+    assert np.array_equal(files["chains"], Cn + rows)
+    assert np.array_equal(files["position"], st.position.numpy()[rows]) and files["position"].itemsize == esize
+    assert np.array_equal(files["potential_energy_grad"], st.potential_energy_grad.numpy()[rows])
+    assert np.array_equal(files["num_doublings"], info.num_doublings.numpy()) and np.array_equal(files["is_turning"], info.is_turning.numpy())
+    assert np.array_equal(files["counters"], [123456789012, 4096, 32, Cn * 32])
+    with pytest.raises(ValueError):
+        bench.write_outputs(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_BYTES // 8 + 1)})
+
+
 def test_elementwise_roofline_arithmetic():
     """The HBM roofline of the tick kernel: algorithmic bytes 11 d s C over the measured launch time; the traffic figures
     come from the committed profile table (profiles/r02_traffic.json), never from a constant in bench.py."""
