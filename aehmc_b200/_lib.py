@@ -77,6 +77,11 @@ class Cfg(C.Structure):
                 ("thin", C.c_int32), ("exact_doubling", C.c_int32), ("reserved", C.c_int32)]
 
 
+class GemmGroup(C.Structure):
+    _fields_ = [("A", C.c_void_p), ("lda", C.c_int64), ("B", C.c_void_p), ("ldb", C.c_int64), ("out", C.c_void_p),
+                ("ldo", C.c_int64), ("M", C.c_int64), ("m_dev", C.c_void_p), ("sub", C.c_void_p), ("tri", C.c_int32)]
+
+
 # every symbol include/b200hmc.h declares (tests check the .so exports all of them)
 EXPORTS = [
     "b2h_last_error", "b2h_version", "b2h_ctx_create", "b2h_ctx_destroy", "b2h_ctx_sync",
@@ -84,7 +89,7 @@ EXPORTS = [
     "b2h_is_turning", "b2h_leapfrog", "b2h_termination_update", "b2h_is_iterative_turning",
     "b2h_find_storage_indices", "b2h_hmc_run", "b2h_nuts_run", "b2h_nuts_workspace_bytes",
     "b2h_hmc_workspace_bytes", "b2h_dual_averaging_update", "b2h_welford_update", "b2h_mass_matrix_final",
-    "b2h_philox_fill", "b2h_dense_apply", "b2h_chain_moments", "b2h_chain_autocov", "b2h_tc_gemm_bf16", "b2h_nuts_expand", "b2h_nuts_subtree", "b2h_proposal_update",
+    "b2h_philox_fill", "b2h_dense_apply", "b2h_chain_moments", "b2h_chain_autocov", "b2h_tc_gemm_bf16", "b2h_gemm", "b2h_nuts_expand", "b2h_nuts_subtree", "b2h_proposal_update",
     "b2h_progressive_sampling", "b2h_select_rows", "b2h_user_model_create", "b2h_user_model_create_ad", "b2h_user_model_destroy",
     "b2h_hmc_accept", "b2h_nuts_plan_group", "b2h_welford_pooled_update", "b2h_welford_pooled_workspace_bytes", "b2h_welford_merge",
     "b2h_tick_timer", "b2h_tick_timer_read",

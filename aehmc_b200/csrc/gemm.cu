@@ -16,6 +16,7 @@
 // the device and which would otherwise cost a full launch latency each.  Rows
 // can be gathered (in_rows) and scattered (out_rows) through index lists.
 #include <algorithm>
+#include <climits>
 #include <type_traits>
 #include <stdlib.h>
 
@@ -741,4 +742,42 @@ void launch_dense_apply(cudaStream_t st, const T* A, const T* B, T* out, int M, 
 B2H_INST(float)
 B2H_INST(double)
 
+template <typename T>
+static GemmGroup<T> to_group(const b2h_gemm_group* g) {
+    if (!g) return GemmGroup<T>{nullptr, 0, nullptr, 0, nullptr, 0, 0, nullptr, nullptr, nullptr, nullptr};
+    return GemmGroup<T>{(const T*)g->A, g->lda, (const T*)g->B, g->ldb, (T*)g->out, g->ldo, (int)g->M,
+                        (const int*)g->m_dev, (const T*)g->sub, nullptr, nullptr, g->tri};
+}
+
+template <typename T>
+static void gemm_entry(cudaStream_t st, const b2h_gemm_group* g, int n, int N, int K, int nsplit, i64 split_stride) {
+    launch_gemm_grouped<T>(st, to_group<T>(g), to_group<T>(n > 1 ? g + 1 : nullptr), to_group<T>(n > 2 ? g + 2 : nullptr),
+                           N, K, nsplit, split_stride, 0);
+}
+
 }  // namespace b2h
+
+extern "C" int b2h_gemm(b2h_ctx* ctx, int dtype, const b2h_gemm_group* groups, int32_t n_groups, int64_t N, int64_t K,
+                        int32_t nsplit, int64_t split_stride) {
+    using namespace b2h;
+    if (!ctx) { set_error("null context"); return B2H_ERR_ARG; }
+    if (dtype != B2H_F32 && dtype != B2H_F64) { set_error("bad dtype"); return B2H_ERR_ARG; }
+    if (!groups || n_groups < 1 || n_groups > 3) { set_error("b2h_gemm: n_groups must be in [1, 3]"); return B2H_ERR_ARG; }
+    if (N < 1 || K < 1 || nsplit < 1 || N > INT_MAX || K > INT_MAX) {
+        set_error("b2h_gemm: N, K and nsplit must be in [1, INT_MAX]");
+        return B2H_ERR_ARG;
+    }
+    for (int i = 0; i < n_groups; ++i) {
+        const b2h_gemm_group& g = groups[i];
+        if (g.M < 0 || g.M > INT_MAX || g.lda < K || g.ldb < N || g.ldo < N) {
+            set_error("b2h_gemm: need 0 <= M <= INT_MAX, lda >= K, ldb >= N and ldo >= N");
+            return B2H_ERR_ARG;
+        }
+        if (g.M > 0 && (!g.A || !g.B || !g.out)) { set_error("b2h_gemm: null matrix pointer"); return B2H_ERR_ARG; }
+        if (g.tri < 0 || g.tri > 2) { set_error("b2h_gemm: tri must be 0, 1 or 2"); return B2H_ERR_ARG; }
+    }
+    if (dtype == B2H_F64) gemm_entry<double>(ctx->stream, groups, n_groups, (int)N, (int)K, nsplit, split_stride);
+    else gemm_entry<float>(ctx->stream, groups, n_groups, (int)N, (int)K, nsplit, split_stride);
+    B2H_LAUNCH_CHECK();
+    return 0;
+}

@@ -369,6 +369,21 @@ int b2h_chain_moments(b2h_ctx*, int dtype, const void* draws, int64_t T, int64_t
 int b2h_tc_gemm_bf16(b2h_ctx*, const void* A, int64_t lda, const void* B, int64_t ldb, float* out, int64_t M, int64_t N,
                      int64_t K, int32_t pieces, int64_t piece_rows, int64_t ldo, int32_t nsplit, int64_t split_stride);
 
+/* One problem of a grouped dense contraction (b2h_gemm).  A [M x K] (pitch lda), B [K x N] (pitch ldb) and out
+ * (pitch ldo) share the dtype of the call.  m_dev: optional device-side row count (rows r < min(M, *m_dev) are
+ * computed).  sub: optional [K] vector subtracted from every row of A.  tri: B is 1 upper- / 2 lower-triangular
+ * (the FP64 tensor path then skips the zero k-range of each column tile), 0 general. */
+typedef struct {
+    const void* A; int64_t lda; const void* B; int64_t ldb; void* out; int64_t ldo;
+    int64_t M; const int32_t* m_dev; const void* sub; int32_t tri;
+} b2h_gemm_group;
+
+/* The dense contraction behind b2h_dense_apply, the correlated-Gaussian gradient, the momentum contractions of the
+ * dense-metric engine and the pooled second moment, exposed for testing: for each of the 1..3 groups,
+ * out + s * split_stride (s < nsplit) = the slice-s split-K partial of (A - sub) . B for rows r < min(M, *m_dev). */
+int b2h_gemm(b2h_ctx*, int dtype, const b2h_gemm_group* groups, int32_t n_groups, int64_t N, int64_t K, int32_t nsplit,
+             int64_t split_stride);
+
 /* Per-chain mean[C x d] and biased autocovariance acov[C x d x (max_lag+1)] (divided by T, the convention of the
  * arviz.ess the reference's tests use, tests/test_hmc.py:158-167) of draws [T][C][d]; building blocks of ESS. */
 int b2h_chain_autocov(b2h_ctx*, int dtype, const void* draws, int64_t T, int64_t C, int64_t d, int32_t max_lag,

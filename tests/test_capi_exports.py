@@ -45,13 +45,13 @@ def test_struct_layouts_match_header_sizes(tmp_path):
     if shutil.which("gcc") is None:
         pytest.skip("needs gcc")
     src = tmp_path / "sz.c"
-    src.write_text('#include <stdio.h>\n#include "b200hmc.h"\nint main(){printf("%zu %zu %zu %zu %zu %zu\\n", '
+    src.write_text('#include <stdio.h>\n#include "b200hmc.h"\nint main(){printf("%zu %zu %zu %zu %zu %zu %zu\\n", '
                    'sizeof(b2h_model), sizeof(b2h_metric), sizeof(b2h_rng), sizeof(b2h_diag), sizeof(b2h_adapt), '
-                   'sizeof(b2h_cfg)); return 0;}\n')
+                   'sizeof(b2h_cfg), sizeof(b2h_gemm_group)); return 0;}\n')
     exe = tmp_path / "sz"
     subprocess.check_call(["gcc", "-I", os.path.join(ROOT, "include"), str(src), "-o", str(exe)])
     sizes = [int(x) for x in subprocess.check_output([str(exe)]).split()]
-    mine = [ctypes.sizeof(getattr(_lib, n)) for n in ("Model", "Metric", "Rng", "Diag", "Adapt", "Cfg")]
+    mine = [ctypes.sizeof(getattr(_lib, n)) for n in ("Model", "Metric", "Rng", "Diag", "Adapt", "Cfg", "GemmGroup")]
     assert mine == sizes
 
 

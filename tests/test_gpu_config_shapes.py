@@ -50,13 +50,36 @@ def _gpu_nuts(ab, model, imm, q0, eps, draws, T, **kw):
 def test_c2_shape_dense_d1000_cta_per_chain(ab):
     """BASELINE configs[1] shape: d = 1000, dense metric, one CTA per chain, 8 chains x 2 transitions.
     Tree depth, leapfrog count and flags bit-exact; positions / energies within 1e-10 relative (north star)."""
-    d, Cn, T = 1000, 8, 2
+    _c2_parity(ab, 8)
+
+
+def test_c2_shape_dense_d1000_4096_chains(ab):
+    """The same at the 4096 chains of the c2 workload: the dense contractions at tile width 112, and the momentum
+    contractions of hundreds of restarting chains walking several row tiles per CTA.  The engine runs all 4096 chains;
+    16 of them (tile edges and seeded random ones) are replayed through the oracle."""
+    _c2_parity(ab, 4096)
+
+
+def _c2_parity(ab, Cn):
+    d, T = 1000, 2
     cov, prec = bench.make_dense_problem(d)
     q0 = bench.initial_positions("dense", Cn, d, 0)
     draws = parity.random_draws(np.random.default_rng(1000), Cn, T, d)
-    ref = parity.oracle_nuts(o_models.CorrelatedGaussian(np.zeros(d), prec), q0, 0.25, cov, draws, T)
     model = ab.models.CorrelatedGaussian(np.zeros(d), prec)
     got = _gpu_nuts(ab, model, cov, q0, 0.25, draws, T, group=256)
+    idx = np.arange(Cn)
+    if Cn > 8:
+        edges = [0, 1, 127, 128, 129, Cn // 2 - 1, Cn - 2, Cn - 1]
+        rest = np.setdiff1d(np.arange(Cn), edges)
+        idx = np.sort(np.concatenate([edges, np.random.default_rng(Cn).choice(rest, 8, replace=False)]))
+        # every chain queues the momentum of its next transition on the tick its current one starts: all Cn on the
+        # first tick, then the chains whose first transition took the same number of leapfrog steps together
+        first = got["stats"][0, :, 2].astype(np.int64)
+        print(f"\nc2 shape, {Cn} chains: momentum contractions of {Cn} restarting chains on the first tick, "
+              f"at most {np.bincount(first).max()} on one later tick")
+        got = {k: (v[:, idx] if k in ("draws", "stats") else v[idx]) for k, v in got.items()}
+    sub = {k: v[idx] for k, v in draws.items()}
+    ref = parity.oracle_nuts(o_models.CorrelatedGaussian(np.zeros(d), prec), q0[idx], 0.25, cov, sub, T)
     parity.assert_nuts_parity(got, ref, rtol=1e-10, atol=1e-10, what="c2 shape")
     assert ref["n_leapfrog"].min() >= 3                      # real trees, not one-step transitions
     np.testing.assert_allclose(got["draws"], ref["draws"], rtol=1e-10, atol=1e-10)

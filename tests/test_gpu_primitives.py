@@ -280,6 +280,7 @@ def test_dense_apply(ab):
     for (Cn, d), dt, tol in (((37, 19), torch.float64, 1e-13), ((300, 257), torch.float64, 1e-13),
                              ((260, 1000), torch.float64, 1e-13), ((64, 112), torch.float64, 1e-13),
                              ((129, 96), torch.float64, 1e-13), ((513, 250), torch.float64, 1e-13),
+                             ((4096, 1000), torch.float64, 1e-13), ((131072, 128), torch.float64, 1e-13),
                              ((130, 128), torch.float32, 1e-5)):
         a = rng.standard_normal((Cn, d)); m = rng.standard_normal((d, d))
         ta, tm = torch.tensor(a, dtype=dt, device="cuda"), torch.tensor(m, dtype=dt, device="cuda")
