@@ -1258,6 +1258,20 @@ static int tc_launch(cudaStream_t st, const void* A, long long lda, const void* 
                      int K, int pieces, int piece_rows, int ldo, int nsplit, long long split_stride, tc::Epilogue ep,
                      int a_blocked = 0, int* resident_tiles_per_cta = nullptr) {
     using namespace tc;
+    // checked before anything is launched: a split plane stride that is not a multiple of four floats misaligns the
+    // epilogue's float4 stores, and a short pitch or piece makes the TMA boxes read another row's (or piece's) data
+    if (M < 1 || N < 1 || K < 1 || pieces < 1 || piece_rows < M) {
+        set_error("tc_gemm: M, N, K and pieces must be positive and piece_rows >= M");
+        return B2H_ERR_ARG;
+    }
+    const bool short_a = a_blocked ? (long long)piece_rows < (long long)((K + BN - 1) / BN) * ((M + BM - 1) / BM) * BM
+                                   : lda < K;
+    if (short_a || ldb < K) { set_error("tc_gemm: the A or B rows do not hold K elements"); return B2H_ERR_ARG; }
+    if (ep.mode == 0 && ldo < N) { set_error("tc_gemm: ldo must be >= N"); return B2H_ERR_ARG; }
+    if (ep.mode == 0 && nsplit > 1 && (split_stride % 4 || split_stride < (long long)(M - 1) * ldo + N)) {
+        set_error("tc_gemm: split_stride must be a multiple of 4 and hold an M x N plane");
+        return B2H_ERR_ARG;
+    }
     if ((lda * 2) % 16 || (ldb * 2) % 16 || ((uintptr_t)A & 15) || ((uintptr_t)B & 15) || ((uintptr_t)out & 15) || ldo % 4) {
         set_error("tc_gemm: operands must be 16-byte aligned with 16-byte row pitches");
         return B2H_ERR_ARG;
@@ -1426,11 +1440,54 @@ int logistic_fused_planes(int M, int N) {
 
 }  // namespace b2h
 
+// the kernels index with int: sizes above INT_MAX would wrap
+static bool ints_fit(std::initializer_list<int64_t> v) {
+    for (int64_t x : v)
+        if (x < 0 || x > 0x7fffffff) { b2h::set_error("tc_gemm: size out of range"); return false; }
+    return true;
+}
+
 extern "C" int b2h_tc_gemm_bf16(b2h_ctx* ctx, const void* A, int64_t lda, const void* B, int64_t ldb, float* out, int64_t M,
                                 int64_t N, int64_t K, int32_t pieces, int64_t piece_rows, int64_t ldo, int32_t nsplit,
                                 int64_t split_stride) {
     if (!ctx) { b2h::set_error("null context"); return B2H_ERR_ARG; }
+    // the TMA row coordinate of the last piece, p * piece_rows + row, is an int as well
+    if (!ints_fit({M, N, K, piece_rows, ldo}) || !ints_fit({(int64_t)pieces * piece_rows})) return B2H_ERR_ARG;
     int rc = b2h::tc_gemm(ctx->stream, A, lda, B, ldb, out, (int)M, (int)N, (int)K, pieces, (int)piece_rows, (int)ldo,
                           nsplit, split_stride);
+    return rc < 0 ? rc : 0;
+}
+
+extern "C" int b2h_tc_logistic_residual(b2h_ctx* ctx, const void* A, int64_t lda, const void* B, int64_t ldb, int64_t M,
+                                        int64_t N, int64_t K, int32_t pieces, int64_t piece_rows, const float* y, void* R,
+                                        int64_t r_piece_stride, double* upart, int32_t* tiles_per_cta) {
+    if (!ctx || !y || !R || !upart || !tiles_per_cta) { b2h::set_error("null argument"); return B2H_ERR_ARG; }
+    if (!ints_fit({M, N, K, piece_rows}) || !ints_fit({(int64_t)pieces * piece_rows})) return B2H_ERR_ARG;
+    const int64_t tile_elems = (int64_t)b2h::tc::BM * b2h::tc::BN;
+    if (M > 0 && N > 0 && r_piece_stride < (N + b2h::tc::BN - 1) / b2h::tc::BN * ((M + b2h::tc::BM - 1) / b2h::tc::BM) * tile_elems) {
+        b2h::set_error("tc_logistic_residual: r_piece_stride does not hold the tile-blocked M x N residual");
+        return B2H_ERR_ARG;
+    }
+    if (r_piece_stride % 8 || ((uintptr_t)y & 15)) {     // 16-byte stores of the pieces, 16-byte loads of y
+        b2h::set_error("tc_logistic_residual: r_piece_stride must be a multiple of 8 and y 16-byte aligned");
+        return B2H_ERR_ARG;
+    }
+    int per = 0;
+    int rc = b2h::tc_gemm_logistic(ctx->stream, A, lda, B, ldb, (int)M, (int)N, (int)K, pieces, (int)piece_rows, y, R,
+                                   r_piece_stride, upart, &per);
+    if (rc < 0) return rc;
+    *tiles_per_cta = per;
+    return 0;
+}
+
+extern "C" int b2h_tc_gemm_blocked_bf16(b2h_ctx* ctx, const void* R, int64_t r_piece_stride, const void* B, int64_t ldb,
+                                        float* out, int64_t M, int64_t N, int64_t K, int32_t pieces, int64_t ldo,
+                                        int32_t nsplit, int64_t split_stride) {
+    if (!ctx) { b2h::set_error("null context"); return B2H_ERR_ARG; }
+    if (!ints_fit({M, N, K, ldo, r_piece_stride / b2h::tc::BN}) || !ints_fit({(int64_t)pieces * (r_piece_stride / b2h::tc::BN)}))
+        return B2H_ERR_ARG;
+    if (r_piece_stride % b2h::tc::BN) { b2h::set_error("tc_gemm_blocked: r_piece_stride must be a multiple of 128"); return B2H_ERR_ARG; }
+    int rc = b2h::tc_gemm_blocked_a(ctx->stream, R, r_piece_stride, B, ldb, out, (int)M, (int)N, (int)K, pieces, (int)ldo,
+                                    nsplit, split_stride);
     return rc < 0 ? rc : 0;
 }

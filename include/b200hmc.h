@@ -365,9 +365,29 @@ int b2h_chain_moments(b2h_ctx*, int dtype, const void* draws, int64_t T, int64_t
 
 /* tcgen05/TMA contraction used by the logistic tensor-core path, exposed for testing:
  * out[z][M x N] (fp32, row pitch ldo, plane stride split_stride) = sum_{p<pieces} A[p*piece_rows + m][k] * B[n][k]
- * with A [pieces*piece_rows x K] and B [N x K] bf16, K contiguous, 16-byte aligned pitches; split-K over z. */
+ * with A [pieces*piece_rows x K] and B [N x K] bf16, K contiguous, 16-byte aligned pitches; split-K over z.
+ * Plane z sums the k-blocks of 64 [z * kb_per, (z + 1) * kb_per), kb_per = ceil(kb / min(nsplit, kb)) with
+ * kb = ceil(K / 64); ceil(kb / kb_per) planes are written.  B2H_ERR_ARG (nothing launched) unless M, N, K, pieces >= 1,
+ * piece_rows >= M, lda, ldb >= K, ldo >= N and, when nsplit > 1, split_stride is a multiple of 4 that is at least
+ * (M - 1) * ldo + N. */
 int b2h_tc_gemm_bf16(b2h_ctx*, const void* A, int64_t lda, const void* B, int64_t ldb, float* out, int64_t M, int64_t N,
                      int64_t K, int32_t pieces, int64_t piece_rows, int64_t ldo, int32_t nsplit, int64_t split_stride);
+/* The first product of the two-kernel logistic gradient, exposed for testing: S = sum_p A_p . B^T (as above, one
+ * plane) never leaves the SM; the epilogue writes r = sigmoid(S) - y[N] as three bf16 pieces r = p0 + p1 + p2 into R,
+ * tile-blocked: piece p, column tile t, row tile u at R + p * r_piece_stride + (t * ceil(M / 128) + u) * 128 * 128,
+ * 128 x 128 row-major (columns >= N of rows < M hold 0; rows >= M are not written).  R 1024-byte aligned, y 16-byte
+ * aligned.  upart receives the fp64 partial sums of softplus(s) - y s per row: *tiles_per_cta == 0: [column tile][4][M];
+ * *tiles_per_cta > 0: [CTA][4][M], CTA b covering the tiles [b, b + 1) * tiles_per_cta of the (row tile, column tile)
+ * grid, column tile fastest.  upart must hold 4 * max(ceil(N / 128), SM count) * M doubles. */
+int b2h_tc_logistic_residual(b2h_ctx*, const void* A, int64_t lda, const void* B, int64_t ldb, int64_t M, int64_t N,
+                             int64_t K, int32_t pieces, int64_t piece_rows, const float* y, void* R, int64_t r_piece_stride,
+                             double* upart, int32_t* tiles_per_cta);
+/* The second product of the two-kernel logistic gradient, exposed for testing: out[z][M x N] = sum_p R_p . B^T (split-K
+ * planes as in b2h_tc_gemm_bf16, k-blocks of 64) with R in the tile-blocked layout of b2h_tc_logistic_residual
+ * (K = data rows, r_piece_stride >= ceil(K / 128) * ceil(M / 128) * 128 * 128, a multiple of 128), B [N x K] bf16. */
+int b2h_tc_gemm_blocked_bf16(b2h_ctx*, const void* R, int64_t r_piece_stride, const void* B, int64_t ldb, float* out,
+                             int64_t M, int64_t N, int64_t K, int32_t pieces, int64_t ldo, int32_t nsplit,
+                             int64_t split_stride);
 
 /* One problem of a grouped dense contraction (b2h_gemm).  A [M x K] (pitch lda), B [K x N] (pitch ldb) and out
  * (pitch ldo) share the dtype of the call.  m_dev: optional device-side row count (rows r < min(M, *m_dev) are

@@ -7,6 +7,7 @@ import pytest
 
 import parity
 from oracle import models as o_models
+from tc_dispatch import tc_plan
 
 pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
@@ -41,13 +42,12 @@ def test_tc_gemm_matches_exact_reference(ab, M, N, K, pieces, nsplit):
     A = torch.randn((pieces * M, K), device="cuda", generator=g).bfloat16()
     B = torch.randn((N, K), device="cuda", generator=g).bfloat16()
     out = _tc_gemm(A, B, M, N, K, pieces, M, nsplit)
-    planes = out.shape[0]
-    got = torch.nan_to_num(out, nan=float("nan")).double()
+    planes = tc_plan(M, N, K, pieces, nsplit)["planes"]       # the split clamping of the host dispatch
+    got = out.double()
     ref = sum(A[p * M:(p + 1) * M].double() @ B.double().T for p in range(pieces))
-    # which planes were written: kernel returns <= nsplit planes; unwritten planes stay NaN
-    written = [z for z in range(planes) if not torch.isnan(got[z]).any()]
-    assert len(written) >= 1
-    total = sum(got[z] for z in written)
+    assert not torch.isnan(got[:planes]).any(), "a plane the dispatch writes was left unwritten"
+    assert torch.isnan(got[planes:]).all(), "a plane beyond the dispatch's count was written"
+    total = got[:planes].sum(0)
     scale = (A.double().abs().max() * B.double().abs().max() * K * pieces).item()
     assert (total - ref).abs().max().item() < 2e-6 * scale
 
