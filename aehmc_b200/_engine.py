@@ -136,6 +136,7 @@ def run(kind, model, metric, srng, state, step_size, *, n_transitions=1, max_num
                              C.c_int32(n_transitions), C.byref(diag), backend.ptr(draws), backend.ptr(stats),
                              C.c_int32(store_draws), backend.ptr(counters), backend.ptr(ws), C.c_int64(ws.numel()))
     _lib.check(rc)
+    model.check_tape()
     del keep
     srng.advance(n_transitions)
     new_state = IntegratorState(q, p, U, g)

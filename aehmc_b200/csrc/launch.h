@@ -101,7 +101,8 @@ int tc_logistic_fused16(cudaStream_t st, const void* beta_pieces, const void* X1
 
 // user_model.cu (NVRTC-compiled user log-density, thread per chain)
 template <typename T>
-int user_potential_and_grad(b2h_ctx* ctx, const b2h_model* m, const T* q, T* U, T* g, i64 C);
+int user_potential_and_grad(b2h_ctx* ctx, const b2h_model* m, const T* q, T* U, T* g, i64 C, void* ws, i64 ws_bytes);
+i64 user_workspace_bytes(const b2h_model* m, int dtype, i64 C);
 
 // engine_kernels.cu
 int nuts_run_impl(b2h_ctx* ctx, const b2h_model* model, const b2h_metric* metric, const b2h_rng* rng,

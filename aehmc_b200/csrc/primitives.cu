@@ -74,7 +74,7 @@ int potential_and_grad_impl(b2h_ctx* ctx, const b2h_model* model, const T* q, T*
         case B2H_MODEL_LOGISTIC:
             return logistic_potential_and_grad<T>(ctx, model, q, U, g, C, ws, ws_bytes, 0);
         case B2H_MODEL_USER:
-            return user_potential_and_grad<T>(ctx, model, q, U, g, C);
+            return user_potential_and_grad<T>(ctx, model, q, U, g, C, ws, ws_bytes);
         default:
             set_error("unknown model kind");
             return B2H_ERR_ARG;
@@ -88,6 +88,7 @@ template int potential_and_grad_impl<double>(b2h_ctx*, const b2h_model*, const d
 
 i64 potential_workspace_bytes_impl(const b2h_model* m, int dtype, i64 C) {
     if (m->kind == B2H_MODEL_LOGISTIC) return logistic_workspace_bytes(m, dtype, C);
+    if (m->kind == B2H_MODEL_USER) return user_workspace_bytes(m, dtype, C);
     return 0;
 }
 

@@ -49,6 +49,7 @@ def velocity_verlet(potential_fn, kinetic_energy_fn):
                                     backend.ptr(p), backend.ptr(U), backend.ptr(g), backend.ptr(eps),
                                     backend.ptr(dirs), C.c_int32(n_steps), C.c_int64(Cn), backend.ptr(w),
                                     C.c_int64(w.numel())))
+        model.check_tape()
         return IntegratorState(q, p, U, g)
 
     one_step.model = model

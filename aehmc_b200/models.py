@@ -36,6 +36,16 @@ class Model:
     # -- hmc.new_state (reference hmc.py:16-40) ----------------------------------------------------
     def potential_and_grad(self, q):
         """U[C], dU/dq[C,d] for positions q[C,d]."""
+        U, g = self._evaluate(q)
+        self.check_tape()
+        return U, g
+
+    def check_tape(self):
+        """Raise if a chain evaluated since the last check needed more tape than a reverse-mode user model holds (its
+        U was +inf and its gradient 0).  Called after every call that evaluates the model; a no-op for every other
+        model."""
+
+    def _evaluate(self, q):
         q = backend.as_device(q, self.dtype, self.device)
         if q.ndim != 2 or q.shape[1] != self.dim:
             raise ValueError(f"position must be [chains, {self.dim}], got {tuple(q.shape)}")
@@ -182,17 +192,28 @@ class UserModel(Model):
         __device__ S log_density(const S* q, int d, const T* data);                 // returns logprob
 
     written with ordinary arithmetic and exp / log / log1p / sqrt / tanh / sin / cos / square / pow / softplus: the
-    gradient then comes from forward-mode dual numbers (the role of ``aesara.grad``; O(dim) per operation, dim <= 64).
-    It is compiled once with NVRTC for sm_100a (``b2h_user_model_create[_ad]``) and evaluated one thread per chain;
+    gradient then comes from automatic differentiation (the role of ``aesara.grad``).  Up to dim 64 it is forward mode,
+    dual numbers carrying all dim partials (O(dim) per operation); above, reverse mode: each chain records a tape of
+    its operations in the workspace and one reverse sweep gives the gradient (O(1) per operation, dim <= 4096).  The
+    tape capacity is probed once here, by evaluating q = 0; a density whose operation count depends on q must pass
+    ``tape_nodes`` (nodes per chain) instead.  A chain that needs more raises ``B200HMCError`` after the call that
+    evaluated it.  It is compiled once with NVRTC for sm_100a (``b2h_user_model_create[_ad|_rev]``) and evaluated one
+    thread per chain;
     the sampler runs it in split mode (one gradient launch per leapfrog tick).  ``data`` is an optional flat array of
     constants handed to the function in the model's dtype.  ``host_fn(q[d]) -> (U, g)`` is an optional NumPy
     counterpart (used by the tests as the oracle's model); it is never called by the sampler."""
     kind = _lib.MODEL_USER
+    FORWARD_MAX_DIM = 64          # autodiff: forward mode up to this dim, reverse mode above
 
-    def __init__(self, source, dim, data=None, dtype=torch.float64, device=None, host_fn=None, autodiff=False):
+    def __init__(self, source, dim, data=None, dtype=torch.float64, device=None, host_fn=None, autodiff=False,
+                 tape_nodes=None):
         super().__init__(dtype, device)
         self.dim = int(dim)
         self.autodiff = bool(autodiff)
+        self.reverse = self.autodiff and self.dim > self.FORWARD_MAX_DIM
+        if tape_nodes is not None and not self.reverse:
+            raise ValueError(f"tape_nodes applies to reverse-mode models (autodiff=True, dim > {self.FORWARD_MAX_DIM})")
+        self.tape_nodes = 0
         self.source = str(source)
         self.host_fn = host_fn
         self.data = None if data is None else backend.as_device(np.asarray(data, dtype=np.float64).ravel(), self.dtype,
@@ -200,12 +221,32 @@ class UserModel(Model):
         lib = _lib.load()
         with torch.cuda.device(self.device):
             handle = C.c_void_p()
-            if self.autodiff:
+            if self.reverse:
+                _lib.check(lib.b2h_user_model_create_rev(self.source.encode(), C.c_int32(self.dim), C.byref(handle)))
+            elif self.autodiff:
                 _lib.check(lib.b2h_user_model_create_ad(self.source.encode(), C.c_int32(self.dim), C.byref(handle)))
             else:
                 _lib.check(lib.b2h_user_model_create(self.source.encode(), C.byref(handle)))
         self._handle = handle
         self._lib = lib
+        if self.reverse:
+            if tape_nodes is None:
+                self._evaluate(torch.zeros((1, self.dim), dtype=self.dtype, device=self.device))
+                tape_nodes = self._tape_needed()
+            _lib.check(lib.b2h_user_model_set_tape_nodes(handle, C.c_int64(int(tape_nodes))))
+            self.tape_nodes = int(tape_nodes)
+
+    def _tape_needed(self):
+        n = C.c_int64()
+        _lib.check(self._lib.b2h_user_model_tape_needed(backend.context(self.device), self._handle, C.byref(n)))
+        return n.value
+
+    def check_tape(self):
+        if self.reverse:
+            n = self._tape_needed()
+            if n > self.tape_nodes:
+                raise _lib.B200HMCError(f"reverse-mode user model: a chain needed {n} tape nodes, the capacity is "
+                                        f"{self.tape_nodes} (pass tape_nodes >= {n} to UserModel)")
 
     def struct(self):
         return _lib.Model(self.kind, self.dim, 0, self._handle.value, None if self.data is None else self.data.data_ptr(),

@@ -117,6 +117,7 @@ def dynamic_integration(srng, integrator, kinetic_energy, update_termination_sta
         _lib.check(lib.b2h_nuts_subtree(backend.context(dev), C.byref(m), C.byref(mt), C.byref(rng), C.byref(cfg),
                                         C.byref(sub), backend.ptr(eps), C.c_int64(Cn), backend.ptr(w),
                                         C.c_int64(w.numel())))
+        model.check_tape()
         del keep
         srng.advance(1)
         return (ProposalState(prop, energy, weight, slpa), st, msum, TerminationState(mck, sck, imin, imax),
@@ -180,6 +181,7 @@ def multiplicative_expansion(srng, trajectory_integrator, uturn_check_fn, max_nu
         _lib.check(lib.b2h_nuts_expand(backend.context(dev), C.byref(m), C.byref(mt), C.byref(rng), C.byref(cfg),
                                        C.byref(tree), backend.ptr(eps), C.c_int64(Cn), C.byref(diag), backend.ptr(w),
                                        C.c_int64(w.numel())))
+        model.check_tape()
         del keep
         srng.advance(1)
         h = lambda t: t.unsqueeze(0)

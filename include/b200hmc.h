@@ -197,6 +197,31 @@ int b2h_user_model_create(const char* cuda_source, b2h_user_model** out);
  * gradient comes from forward-mode dual numbers S = Dual<T, dim> (the role of aesara.grad; O(dim) per operation,
  * dim <= 64). */
 int b2h_user_model_create_ad(const char* cuda_source, int32_t dim, b2h_user_model** out);
+/* Same log_density source, differentiated in reverse mode: S = Var<T> holds the value (.v, as in Dual, so a source
+ * that branches on q[i].v compiles in both modes) and a node id.  One evaluation records a tape per chain; one reverse
+ * sweep over it gives the gradient, at a cost proportional to the number of operations whatever dim is.  U is
+ * bit-identical to the forward mode's; the gradient differs only in the order its terms are summed.
+ * 1 <= dim <= B2H_USER_REV_MAX_DIM (the inputs are a per-thread array of dim Vars in local memory).
+ *
+ * The tape lives in the workspace of every call that evaluates the model (b2h_potential_and_grad, b2h_leapfrog, the
+ * engine and the tree builders size it through b2h_potential_workspace_bytes).  With N = the tape capacity in nodes
+ * per chain, pitch = C rounded up to a multiple of 32 and E = sizeof(T) (8 for B2H_F64, 4 for B2H_F32):
+ *     bytes = 256 + 2 * R(N * pitch * 4) + 2 * R(N * pitch * E) + R((dim + N) * pitch * E),   R(x) = x rounded up to 256
+ * (two int32 operand ids and two partials per node, adjoints of the inputs and the nodes; 8 + 3E bytes per node).
+ * A smaller workspace returns B2H_ERR_WORKSPACE.  Its contents need not be initialised.
+ *
+ * The capacity starts at 0.  A chain that needs more nodes than the capacity still computes its values but gets
+ * U = +inf and g = 0 (the sampler rejects it as a divergence), and the count it needed is recorded on the device:
+ * read it with b2h_user_model_tape_needed after each evaluating call to detect this.  The handle must be used with
+ * contexts on the device that was current at creation (B2H_ERR_ARG otherwise). */
+#define B2H_USER_REV_MAX_DIM 4096
+int b2h_user_model_create_rev(const char* cuda_source, int32_t dim, b2h_user_model** out);
+/* Sets the tape capacity in nodes per chain, 0 <= nodes <= 2^31 - 1 - dim.  The workspace size depends on it: a
+ * workspace sized before the change may be too small afterwards. */
+int b2h_user_model_set_tape_nodes(b2h_user_model* model, int64_t nodes);
+/* *needed = the largest node count any chain of a reverse-mode handle needed since the previous read (0 if none was
+ * evaluated), then resets it.  Copies on the context's stream and synchronises that stream. */
+int b2h_user_model_tape_needed(b2h_ctx* ctx, b2h_user_model* model, int64_t* needed);
 int b2h_user_model_destroy(b2h_user_model* model);
 
 int b2h_potential_and_grad(b2h_ctx*, const b2h_model*, int dtype, const void* q, void* U, void* g, int64_t C,
