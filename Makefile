@@ -13,7 +13,8 @@ LIB       := $(LIBDIR)/libb200hmc.so
 # contraction so that the scalar-metric leapfrog rounds exactly like the reference's
 # compiled graph (a*b then +c); the contraction kernels keep FMA.
 OBJS := $(OBJDIR)/capi.o $(OBJDIR)/engine_kernels.o $(OBJDIR)/engine_fused_f32.o $(OBJDIR)/engine_fused_f64.o \
-        $(OBJDIR)/engine_split_f32.o $(OBJDIR)/engine_split_f64.o $(OBJDIR)/primitives.o $(OBJDIR)/gemm.o $(OBJDIR)/logreg.o $(OBJDIR)/tc_gemm.o $(OBJDIR)/user_model.o $(OBJDIR)/pooled.o
+        $(OBJDIR)/engine_split_f32.o $(OBJDIR)/engine_split_f64.o $(OBJDIR)/primitives.o $(OBJDIR)/gemm.o $(OBJDIR)/logreg.o $(OBJDIR)/tc_gemm.o $(OBJDIR)/user_model.o $(OBJDIR)/pooled.o \
+        $(OBJDIR)/dense_per_chain.o
 HDRS := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) $(wildcard $(CSRC)/*.inl) include/b200hmc.h
 
 all: $(LIB)

@@ -86,6 +86,9 @@ def run(kind, model, metric, srng, state, step_size, *, n_transitions=1, max_num
         raise ValueError("inverse mass matrix and position dimensions differ")
     if metric.kind == _lib.IMM_DIAG_PER_CHAIN and metric.imm.shape[0] != Cn:
         raise ValueError("per-chain inverse mass matrix must be [chains, dim]")
+    if metric.kind == _lib.IMM_DENSE_PER_CHAIN and tuple(metric.imm.shape) != (Cn, d, d):
+        raise ValueError(f"per-chain dense inverse mass matrix must be [chains, dim, dim] = [{Cn}, {d}, {d}], got "
+                         f"{list(metric.imm.shape)}")
     U = backend.as_device(state.potential_energy, dt, dev).clone()
     g = backend.as_device(state.potential_energy_grad, dt, dev).clone()
     p = torch.empty_like(q)

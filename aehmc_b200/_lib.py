@@ -14,7 +14,8 @@ LIB_PATH = os.environ.get("B2H_LIB") or os.path.join(_HERE, "lib", "libb200hmc.s
 
 F32, F64 = 0, 1
 MODEL_IID_GAUSSIAN, MODEL_CORR_GAUSSIAN, MODEL_FUNNEL, MODEL_EIGHT_SCHOOLS, MODEL_LOGISTIC, MODEL_USER = range(6)
-IMM_SCALAR, IMM_DIAG, IMM_DIAG_PER_CHAIN, IMM_DENSE = range(4)
+IMM_SCALAR, IMM_DIAG, IMM_DIAG_PER_CHAIN, IMM_DENSE, IMM_DENSE_PER_CHAIN = range(5)
+DENSE_PER_CHAIN_MAX_DIM = 128   # B2H_DENSE_PER_CHAIN_MAX_DIM
 RNG_PHILOX, RNG_INJECTED = 0, 1
 
 
@@ -89,7 +90,7 @@ EXPORTS = [
     "b2h_is_turning", "b2h_leapfrog", "b2h_termination_update", "b2h_is_iterative_turning",
     "b2h_find_storage_indices", "b2h_hmc_run", "b2h_nuts_run", "b2h_nuts_workspace_bytes",
     "b2h_hmc_workspace_bytes", "b2h_dual_averaging_update", "b2h_welford_update", "b2h_mass_matrix_final",
-    "b2h_philox_fill", "b2h_dense_apply", "b2h_chain_moments", "b2h_chain_autocov", "b2h_tc_gemm_bf16", "b2h_tc_logistic_residual",
+    "b2h_philox_fill", "b2h_dense_apply", "b2h_dense_apply_per_chain", "b2h_dense_factor_per_chain", "b2h_chain_moments", "b2h_chain_autocov", "b2h_tc_gemm_bf16", "b2h_tc_logistic_residual",
     "b2h_tc_gemm_blocked_bf16", "b2h_gemm", "b2h_nuts_expand", "b2h_nuts_subtree", "b2h_proposal_update",
     "b2h_progressive_sampling", "b2h_select_rows", "b2h_user_model_create", "b2h_user_model_create_ad", "b2h_user_model_create_rev",
     "b2h_user_model_set_tape_nodes", "b2h_user_model_tape_needed", "b2h_user_model_destroy",

@@ -13,6 +13,7 @@ constexpr int kRiderSplit = 5;      // split-K slices of the momentum contractio
 struct EnginePlan {
     int G;
     bool dense, split, hmc, per_chain_imm, scalar_imm;
+    bool dense_per_chain;   // B2H_IMM_DENSE_PER_CHAIN: dense (same tick kernels), the metric mat-vecs per chain
     size_t model_ws_off, model_ws_bytes;
 };
 

@@ -53,7 +53,13 @@ static bool model_is_fused(int kind) {
 
 static int make_plan(const b2h_model* model, const b2h_metric* metric, const b2h_cfg* cfg, EnginePlan& pl,
                      long long C = 0, bool free_running = false) {
-    pl.dense = metric->kind == B2H_IMM_DENSE;
+    pl.dense_per_chain = metric->kind == B2H_IMM_DENSE_PER_CHAIN;
+    pl.dense = metric->kind == B2H_IMM_DENSE || pl.dense_per_chain;
+    if (pl.dense_per_chain && (model->dim < 1 || model->dim > B2H_DENSE_PER_CHAIN_MAX_DIM)) {
+        set_error("a per-chain dense metric needs 1 <= d <= " + std::to_string(B2H_DENSE_PER_CHAIN_MAX_DIM) +
+                  " (B2H_DENSE_PER_CHAIN_MAX_DIM); for larger d adapt one shared dense matrix (pooled=True)");
+        return B2H_ERR_ARG;
+    }
     pl.per_chain_imm = metric->kind == B2H_IMM_DIAG_PER_CHAIN;
     pl.scalar_imm = metric->kind == B2H_IMM_SCALAR;
     pl.split = pl.dense || !model_is_fused(model->kind);
@@ -102,7 +108,8 @@ static size_t carve(EngineView<T>& v, char* base, const EnginePlan& pl, const b2
         v.xc = cv.take<T>(n);
         v.mom_p = cv.take<T>(n); v.mom_v = cv.take<T>(n); v.mom_z = cv.take<T>(2 * n);
         v.mom_count = cv.take<int>(4); v.mom_list = cv.take<int>(2 * (size_t)C);
-        v.mom_part = cv.take<T>(2 * (size_t)kRiderSplit * n);
+        // the shared matrix's rider is a split-K contraction; the per-chain one writes its rows directly
+        v.mom_part = pl.dense_per_chain ? nullptr : cv.take<T>(2 * (size_t)kRiderSplit * n);
     }
     v.scratch = cv.take<int>(64);
     if (model_ws_bytes) {

@@ -67,6 +67,25 @@ template <typename T>
 void launch_dense_apply(cudaStream_t st, const T* A, const T* B, T* out, int M, int N, int K, const int* m_dev,
                         const T* sub);
 
+// dense_per_chain.cu: out[m][chain(r)] = in[r] . M[m][chain(r)] for rows r < min(rows, *count), chain(r) = list[r]
+// (identity when list is null); M[m] + c * d * d is chain c's [d x d] matrix, tri[m] as GemmGroup::tri.  One matrix
+// (M[1] = nullptr) or two from the same input row (the momentum rider).
+template <typename T>
+struct PcJob {
+    const T* in;
+    const T* M[2];
+    T* out[2];
+    int tri[2];
+    const int* count;      // optional device-side row count
+    const int* list;       // optional row -> chain list
+    i64 rows;
+    int d;
+};
+template <typename T>
+void launch_dense_pc(cudaStream_t st, const PcJob<T>& job);
+template <typename T>
+void launch_dense_apply_pc(cudaStream_t st, const T* in, const T* M, T* out, i64 C, int d, int tri);
+
 template <typename T>
 void launch_gemm(cudaStream_t st, const T* A, i64 lda, const T* B, i64 ldb, T* out, i64 ldo, int M, int N, int K,
                  const int* m_dev, const T* sub, int nsplit, i64 split_stride);

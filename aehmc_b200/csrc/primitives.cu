@@ -110,6 +110,27 @@ static ImmView imm_view(const b2h_metric* m, i64 d) {
     return v;
 }
 
+static bool is_dense(const b2h_metric* m) { return m->kind == B2H_IMM_DENSE || m->kind == B2H_IMM_DENSE_PER_CHAIN; }
+
+// out = in . M of a dense metric: the shared [d x d] matrix through the dense contraction, per-chain [C x d x d]
+// matrices through the batched per-chain product (tri applies to the latter; the shared path reads M in full)
+template <typename T>
+static void metric_apply(cudaStream_t st, const b2h_metric* m, const T* in, const void* M, T* out, i64 C, int d, int tri) {
+    if (m->kind == B2H_IMM_DENSE_PER_CHAIN) launch_dense_apply_pc<T>(st, in, (const T*)M, out, C, d, tri);
+    else launch_dense_apply<T>(st, in, (const T*)M, out, (int)C, d, d, nullptr, nullptr);
+}
+
+static int check_metric(const b2h_metric* m, i64 d) {
+    if (m->kind != B2H_IMM_DENSE_PER_CHAIN) return 0;
+    if (!m->imm || !m->sqrt_t || !m->chol_t) { set_error("per-chain dense metric needs imm, sqrt_t and chol_t"); return B2H_ERR_ARG; }
+    if (d < 1 || d > B2H_DENSE_PER_CHAIN_MAX_DIM) {
+        set_error("a per-chain dense metric needs 1 <= d <= " + std::to_string(B2H_DENSE_PER_CHAIN_MAX_DIM) +
+                  " (B2H_DENSE_PER_CHAIN_MAX_DIM); for larger d adapt one shared dense matrix (pooled=True)");
+        return B2H_ERR_ARG;
+    }
+    return 0;
+}
+
 template <typename T>
 B2H_DEVINL T imm_at(const ImmView& v, i64 c, int j) {
     if (v.kind == B2H_IMM_SCALAR) return (T)v.scalar;
@@ -279,7 +300,8 @@ static int leapfrog_typed(b2h_ctx* ctx, const b2h_model* model, const b2h_metric
     const int d = model->dim;
     ImmView iv = imm_view(metric, d);
     ModelDev m = to_dev(model);
-    const bool dense = metric->kind == B2H_IMM_DENSE;
+    const bool dense = is_dense(metric);
+    if (int rc = check_metric(metric, d)) return rc;
     const bool fused = !dense && (model->kind == B2H_MODEL_IID_GAUSSIAN || model->kind == B2H_MODEL_FUNNEL ||
                                   model->kind == B2H_MODEL_EIGHT_SCHOOLS);
     if (fused) {
@@ -313,7 +335,7 @@ static int leapfrog_typed(b2h_ctx* ctx, const b2h_model* model, const b2h_metric
     for (int s = 0; s < n_steps; ++s) {
         halfkick_kernel<T><<<eg, eb, 0, st>>>(iv, q, p, g, eps, dir, C, d, dense ? 0 : 1);
         if (dense) {
-            launch_dense_apply<T>(st, p, (const T*)metric->imm, vel, (int)C, d, d, nullptr, nullptr);
+            metric_apply<T>(st, metric, p, metric->imm, vel, C, d, 0);
             drift_kernel<T><<<eg, eb, 0, st>>>(q, vel, eps, dir, C, d);
         }
         int rc = potential_and_grad_impl<T>(ctx, model, q, U, g, C, model_ws, mws);
@@ -764,17 +786,19 @@ int b2h_sample_momentum(b2h_ctx* ctx, const b2h_metric* metric, const b2h_rng* r
     rv.chain_offset = rng->chain_offset; rv.transition_offset = rng->transition_offset;
     rv.n_injected = rng->n_injected; rv.z = rng->z; rv.u_dir = rv.u_biased = rv.u_uniform = rv.u_accept = nullptr;
     ImmView iv = imm_view(metric, d);
-    const bool dense = metric->kind == B2H_IMM_DENSE;
+    const bool dense = is_dense(metric);
+    if (int rc = check_metric(metric, d)) return rc;
+    const int tri = (metric->reserved & 1) ? 2 : 0;          // sqrt_t = L^-1 is lower-triangular
     const i64 n = C * d;
     const int eb = 256, eg = (int)((n + eb - 1) / eb);
     if (dense && (!ws || ws_bytes < n * (i64)dtype_size(dtype))) { set_error("momentum workspace too small"); return B2H_ERR_WORKSPACE; }
     cudaStream_t st = ctx->stream;
     if (dtype == B2H_F64) {
         momentum_kernel<double><<<eg, eb, 0, st>>>(iv, rv, dense ? (double*)ws : (double*)p, C, (int)d, (int)transition, dense);
-        if (dense) launch_dense_apply<double>(st, (const double*)ws, (const double*)metric->sqrt_t, (double*)p, (int)C, (int)d, (int)d, nullptr, nullptr);
+        if (dense) metric_apply<double>(st, metric, (const double*)ws, metric->sqrt_t, (double*)p, C, (int)d, tri);
     } else if (dtype == B2H_F32) {
         momentum_kernel<float><<<eg, eb, 0, st>>>(iv, rv, dense ? (float*)ws : (float*)p, C, (int)d, (int)transition, dense);
-        if (dense) launch_dense_apply<float>(st, (const float*)ws, (const float*)metric->sqrt_t, (float*)p, (int)C, (int)d, (int)d, nullptr, nullptr);
+        if (dense) metric_apply<float>(st, metric, (const float*)ws, metric->sqrt_t, (float*)p, C, (int)d, tri);
     } else { set_error("bad dtype"); return B2H_ERR_ARG; }
     B2H_LAUNCH_CHECK();
     return 0;
@@ -785,16 +809,17 @@ int b2h_kinetic_energy(b2h_ctx* ctx, const b2h_metric* metric, int dtype, const 
     B2H_CHECK_CTX();
     if (!metric || !p || !K) { set_error("bad argument"); return B2H_ERR_ARG; }
     ImmView iv = imm_view(metric, d);
-    const bool dense = metric->kind == B2H_IMM_DENSE;
+    const bool dense = is_dense(metric);
+    if (int rc = check_metric(metric, d)) return rc;
     if (dense && (!ws || ws_bytes < C * d * (i64)dtype_size(dtype))) { set_error("kinetic workspace too small"); return B2H_ERR_WORKSPACE; }
     cudaStream_t st = ctx->stream;
     const int grid = PGeo<32>::grid(C);
     if (dtype == B2H_F64) {
-        if (dense) launch_dense_apply<double>(st, (const double*)p, (const double*)metric->imm, (double*)ws, (int)C, (int)d, (int)d, nullptr, nullptr);
+        if (dense) metric_apply<double>(st, metric, (const double*)p, metric->imm, (double*)ws, C, (int)d, 0);
         if (vec_ok(iv, d, dtype, {p, dense ? ws : nullptr})) kinetic_vec_kernel<double><<<grid, 128, 0, st>>>(iv, (const double*)p, dense ? (const double*)ws : nullptr, (double*)K, C, (int)d);
         else kinetic_kernel<double><<<grid, 128, 0, st>>>(iv, (const double*)p, dense ? (const double*)ws : nullptr, (double*)K, C, (int)d);
     } else if (dtype == B2H_F32) {
-        if (dense) launch_dense_apply<float>(st, (const float*)p, (const float*)metric->imm, (float*)ws, (int)C, (int)d, (int)d, nullptr, nullptr);
+        if (dense) metric_apply<float>(st, metric, (const float*)p, metric->imm, (float*)ws, C, (int)d, 0);
         if (vec_ok(iv, d, dtype, {p, dense ? ws : nullptr})) kinetic_vec_kernel<float><<<grid, 128, 0, st>>>(iv, (const float*)p, dense ? (const float*)ws : nullptr, (float*)K, C, (int)d);
         else kinetic_kernel<float><<<grid, 128, 0, st>>>(iv, (const float*)p, dense ? (const float*)ws : nullptr, (float*)K, C, (int)d);
     } else { set_error("bad dtype"); return B2H_ERR_ARG; }
@@ -807,7 +832,8 @@ int b2h_is_turning(b2h_ctx* ctx, const b2h_metric* metric, int dtype, const void
     B2H_CHECK_CTX();
     if (!metric || !pl || !pr || !ps || !out) { set_error("bad argument"); return B2H_ERR_ARG; }
     ImmView iv = imm_view(metric, d);
-    const bool dense = metric->kind == B2H_IMM_DENSE;
+    const bool dense = is_dense(metric);
+    if (int rc = check_metric(metric, d)) return rc;
     const i64 n = C * d;
     if (dense && (!ws || ws_bytes < 2 * n * (i64)dtype_size(dtype))) { set_error("is_turning workspace too small"); return B2H_ERR_WORKSPACE; }
     cudaStream_t st = ctx->stream;
@@ -815,16 +841,16 @@ int b2h_is_turning(b2h_ctx* ctx, const b2h_metric* metric, int dtype, const void
     if (dtype == B2H_F64) {
         double* vl = dense ? (double*)ws : nullptr; double* vr = dense ? vl + n : nullptr;
         if (dense) {
-            launch_dense_apply<double>(st, (const double*)pl, (const double*)metric->imm, vl, (int)C, (int)d, (int)d, nullptr, nullptr);
-            launch_dense_apply<double>(st, (const double*)pr, (const double*)metric->imm, vr, (int)C, (int)d, (int)d, nullptr, nullptr);
+            metric_apply<double>(st, metric, (const double*)pl, metric->imm, vl, C, (int)d, 0);
+            metric_apply<double>(st, metric, (const double*)pr, metric->imm, vr, C, (int)d, 0);
         }
         if (vec_ok(iv, d, dtype, {pl, pr, ps, vl, vr})) turning_vec_kernel<double><<<grid, 128, 0, st>>>(iv, (const double*)pl, (const double*)pr, (const double*)ps, vl, vr, out, C, (int)d);
         else turning_kernel<double><<<grid, 128, 0, st>>>(iv, (const double*)pl, (const double*)pr, (const double*)ps, vl, vr, out, C, (int)d);
     } else if (dtype == B2H_F32) {
         float* vl = dense ? (float*)ws : nullptr; float* vr = dense ? vl + n : nullptr;
         if (dense) {
-            launch_dense_apply<float>(st, (const float*)pl, (const float*)metric->imm, vl, (int)C, (int)d, (int)d, nullptr, nullptr);
-            launch_dense_apply<float>(st, (const float*)pr, (const float*)metric->imm, vr, (int)C, (int)d, (int)d, nullptr, nullptr);
+            metric_apply<float>(st, metric, (const float*)pl, metric->imm, vl, C, (int)d, 0);
+            metric_apply<float>(st, metric, (const float*)pr, metric->imm, vr, C, (int)d, 0);
         }
         if (vec_ok(iv, d, dtype, {pl, pr, ps, vl, vr})) turning_vec_kernel<float><<<grid, 128, 0, st>>>(iv, (const float*)pl, (const float*)pr, (const float*)ps, vl, vr, out, C, (int)d);
         else turning_kernel<float><<<grid, 128, 0, st>>>(iv, (const float*)pl, (const float*)pr, (const float*)ps, vl, vr, out, C, (int)d);
@@ -874,7 +900,7 @@ int b2h_is_iterative_turning(b2h_ctx* ctx, const b2h_metric* metric, int dtype, 
                              const int64_t* imin, const int64_t* imax, const void* msum, const void* mom, uint8_t* out,
                              int64_t C, int64_t d, int32_t maxd) {
     B2H_CHECK_CTX();
-    if (metric->kind == B2H_IMM_DENSE) { set_error("is_iterative_turning primitive: dense metric not supported (use nuts_run)"); return B2H_ERR_UNSUPPORTED; }
+    if (is_dense(metric)) { set_error("is_iterative_turning primitive: dense metric not supported (use nuts_run)"); return B2H_ERR_UNSUPPORTED; }
     ImmView iv = imm_view(metric, d);
     const int grid = PGeo<32>::grid(C);
     if (vec_ok(iv, d, dtype, {mck, sck, msum, mom})) {

@@ -110,3 +110,36 @@ class PooledWelford:
         shrink = 1e-3 * (5.0 / (n + 5.0))
         out = scaled + shrink * torch.eye(self.d, dtype=torch.float64, device=self.device) if self.full else scaled + shrink
         return out.to(dtype)
+
+
+class PerChainWelford:
+    """Per-chain Welford state of one slow window for dense per-chain adaptation: (mean [C, d], m2 [C, d, d], n [C])
+    in the dtype of the draws, the state of the reference's welford_covariance run once per chain.  ``update`` folds a
+    block of draws [T, C, d] one transition at a time, in order, with the reference's recurrence
+    (``b2h_welford_update``, algorithms.py:166-197, in place); ``final`` applies the shrinkage of
+    mass_matrix.py:103-116 and returns imm [C, d, d]."""
+
+    def __init__(self, num_chains, n_dims, dtype, device):
+        self.C, self.d, self.dtype, self.device = int(num_chains), int(n_dims), dtype, device
+        self.mean = torch.zeros((self.C, self.d), dtype=dtype, device=device)
+        self.m2 = torch.zeros((self.C, self.d, self.d), dtype=dtype, device=device)
+        self.n = torch.zeros(self.C, dtype=torch.int64, device=device)
+
+    def reset(self):
+        self.mean.zero_()
+        self.m2.zero_()
+        self.n.zero_()
+
+    def update(self, draws):
+        x = backend.as_device(draws, self.dtype, self.device)
+        lib, ctx, code = _lib.load(), backend.context(self.device), backend.code(self.dtype)
+        for t in range(x.shape[0]):
+            _lib.check(lib.b2h_welford_update(ctx, code, backend.ptr(x[t]), backend.ptr(self.mean), backend.ptr(self.m2),
+                                              backend.ptr(self.n), C.c_int64(self.C), C.c_int64(self.d), C.c_int32(1)))
+
+    def all_reduce(self):
+        """Nothing to merge: every chain keeps its own statistics."""
+        return self
+
+    def final(self, dtype=None):
+        return covariance_adaptation(True)[2]((self.mean, self.m2, self.n))

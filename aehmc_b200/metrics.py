@@ -2,8 +2,8 @@
 
 ``gaussian_metric(inverse_mass_matrix)`` keeps the reference's contract: a 0-d, 1-d (diagonal)
 or 2-d (dense, shared by all chains) inverse mass matrix, ``ValueError`` above 2-d, and returns
-``(momentum_generator, kinetic_energy, is_turning)``.  A per-chain diagonal matrix (what per-chain
-window adaptation produces) is passed as ``per_chain(imm[C, d])``.
+``(momentum_generator, kinetic_energy, is_turning)``.  One matrix per chain (what per-chain window
+adaptation produces) is passed as ``per_chain(imm[C, d])`` (diagonal) or ``per_chain(imm[C, d, d])`` (dense).
 """
 from __future__ import annotations
 
@@ -16,7 +16,10 @@ from . import _lib, backend
 
 
 class per_chain:
-    """Marks a [chains, dim] tensor as one diagonal inverse mass matrix per chain."""
+    """Marks a tensor as one inverse mass matrix per chain: ``[chains, dim]`` diagonal or ``[chains, dim, dim]``
+    dense (dim <= 128).  A dense one is symmetrised, ``(A + A^T) / 2`` as for a shared matrix, and factored on the
+    device (``b2h_dense_factor_per_chain``, FP64 Cholesky); ``ValueError`` names the chains whose matrix is not
+    positive definite."""
 
     def __init__(self, imm):
         self.imm = imm
@@ -38,9 +41,11 @@ class GaussianMetric:
         self.device = backend.device(device)
         ndim = imm.ndim if isinstance(imm, torch.Tensor) else np.ndim(imm)
         self.scalar, self.imm, self.sqrt_t, self.chol_t = 0.0, None, None, None
-        if pc:
+        if pc and ndim == 3:
+            self._factor_per_chain(backend.as_device(imm, self.dtype, self.device))
+        elif pc:
             if ndim != 2:
-                raise ValueError("per_chain() expects a [chains, dim] tensor")
+                raise ValueError("per_chain() expects a [chains, dim] or [chains, dim, dim] tensor")
             self.kind = _lib.IMM_DIAG_PER_CHAIN
             self.imm = backend.as_device(imm, self.dtype, self.device)
             self.dim = int(self.imm.shape[1])
@@ -69,11 +74,29 @@ class GaussianMetric:
             raise ValueError(f"Expected a mass matrix of dimension 1 (diagonal) or 2, got {ndim}")
         self._ws = backend.Workspace()
 
+    def _factor_per_chain(self, a):
+        Cn, d, d2 = a.shape
+        if d != d2:
+            raise ValueError(f"per_chain() dense matrices must be square, got [{Cn}, {d}, {d2}]")
+        if not 1 <= d <= _lib.DENSE_PER_CHAIN_MAX_DIM:
+            raise ValueError(f"per-chain dense inverse mass matrices need dim <= {_lib.DENSE_PER_CHAIN_MAX_DIM}, got "
+                             f"{d}; adapt one shared dense matrix instead (window_adaptation.run(..., pooled=True))")
+        self.kind, self.dim = _lib.IMM_DENSE_PER_CHAIN, int(d)
+        self.imm, self.sqrt_t, self.chol_t = (torch.empty_like(a) for _ in range(3))
+        info = torch.empty(Cn, dtype=torch.int32, device=self.device)
+        _lib.check(_lib.load().b2h_dense_factor_per_chain(
+            backend.context(self.device), backend.code(self.dtype), backend.ptr(a), backend.ptr(self.imm),
+            backend.ptr(self.sqrt_t), backend.ptr(self.chol_t), backend.ptr(info), C.c_int64(Cn), C.c_int64(d)))
+        bad = torch.nonzero(info).flatten().tolist()
+        if bad:
+            shown = ", ".join(str(c) for c in bad[:8]) + (f" and {len(bad) - 8} more" if len(bad) > 8 else "")
+            raise ValueError(f"per_chain(): the inverse mass matrix is not positive definite for chain(s) {shown}")
+
     def struct(self):
         p = lambda t: None if t is None else t.data_ptr()
-        # flags bit 0: sqrt_t / chol_t are the triangular Cholesky factors built above (b200hmc.h)
-        return _lib.Metric(self.kind, 1 if self.kind == _lib.IMM_DENSE else 0, self.scalar, p(self.imm), p(self.sqrt_t),
-                           p(self.chol_t))
+        # flags bit 0: sqrt_t / chol_t are the triangular Cholesky factors built here (b200hmc.h)
+        dense = self.kind in (_lib.IMM_DENSE, _lib.IMM_DENSE_PER_CHAIN)
+        return _lib.Metric(self.kind, 1 if dense else 0, self.scalar, p(self.imm), p(self.sqrt_t), p(self.chol_t))
 
     def _ws_for(self, n_elems):
         nbytes = n_elems * (8 if self.dtype == torch.float64 else 4) + 512
@@ -88,7 +111,8 @@ def gaussian_metric(inverse_mass_matrix, dtype=None, device=None):
     def momentum_generator(srng, num_chains=None, dim=None, transition=None):
         """p[C, d] = M^{1/2} z (metrics.py:65-68).  Shape comes from the metric when it has one."""
         d = metric.dim or dim
-        Cn = num_chains if num_chains is not None else (metric.imm.shape[0] if metric.kind == _lib.IMM_DIAG_PER_CHAIN else None)
+        per_chain_kind = metric.kind in (_lib.IMM_DIAG_PER_CHAIN, _lib.IMM_DENSE_PER_CHAIN)
+        Cn = num_chains if num_chains is not None else (metric.imm.shape[0] if per_chain_kind else None)
         if d is None or Cn is None:
             raise ValueError("momentum_generator needs num_chains (and dim for a scalar metric)")
         p = torch.empty((Cn, d), dtype=metric.dtype, device=metric.device)

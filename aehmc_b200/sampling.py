@@ -10,8 +10,9 @@ from .integrators import IntegratorState
 from .random import RandomStream
 
 CHECKPOINT_VERSION = 2
+# "per_chain" covers the diagonal [C, d] and the dense [C, d, d] kinds: the shape tells them apart
 _KIND_NAMES = {_lib.IMM_SCALAR: "scalar", _lib.IMM_DIAG: "diag", _lib.IMM_DIAG_PER_CHAIN: "per_chain",
-               _lib.IMM_DENSE: "dense"}
+               _lib.IMM_DENSE: "dense", _lib.IMM_DENSE_PER_CHAIN: "per_chain"}
 
 
 def sample(kernel, state, step_size, inverse_mass_matrix, num_samples, *, num_integration_steps=None,
@@ -69,7 +70,7 @@ def checkpoint(state, srng, step_size, inverse_mass_matrix):
 
 def restore(ckpt, device=None):
     """Inverse of :func:`checkpoint`: returns (state, srng, step_size, inverse_mass_matrix) on ``device``; a
-    per-chain diagonal inverse mass matrix comes back wrapped in ``metrics.per_chain``."""
+    per-chain inverse mass matrix (diagonal [C, d] or dense [C, d, d]) comes back wrapped in ``metrics.per_chain``."""
     if ckpt.get("version") != CHECKPOINT_VERSION:
         raise ValueError(f"unknown checkpoint version {ckpt.get('version')}")
     dev = torch.device("cuda" if device is None else device)

@@ -78,8 +78,16 @@ enum {
     B2H_IMM_SCALAR = 0,         /* 0-d inverse mass matrix, value in .scalar (host)               */
     B2H_IMM_DIAG = 1,           /* imm[d] shared by all chains                                    */
     B2H_IMM_DIAG_PER_CHAIN = 2, /* imm[C x d] (per-chain adaptation)                              */
-    B2H_IMM_DENSE = 3           /* imm[d x d] symmetric, shared; sqrt = mass_matrix_sqrt[d x d]   */
+    B2H_IMM_DENSE = 3,          /* imm[d x d] symmetric, shared; sqrt = mass_matrix_sqrt[d x d]   */
+    B2H_IMM_DENSE_PER_CHAIN = 4 /* imm, sqrt_t, chol_t [C x d x d] row-major, chain c's matrix at c * d * d; each
+                                   chain's triple follows the B2H_IMM_DENSE conventions below (reserved bit 0 too) */
 };
+
+/* Largest d of a B2H_IMM_DENSE_PER_CHAIN metric.  b2h_dense_factor_per_chain keeps a chain's matrix in the shared
+ * memory of one CTA as FP64 (d = 128: 128 KB), and the per-chain metric costs 3 d^2 s bytes per chain (s = dtype size)
+ * plus d^2 s for the per-chain Welford state of its adaptation: 4096 chains at d = 128 in FP64 take 1.6 GB + 0.5 GB.
+ * Larger d (or chains that share one matrix) want the shared B2H_IMM_DENSE kind: window adaptation with pooled = 1. */
+#define B2H_DENSE_PER_CHAIN_MAX_DIM 128
 
 typedef struct {
     int32_t kind;
@@ -144,7 +152,10 @@ typedef struct {
     int64_t* wc_n;              /* [C] */
     int32_t pooled;             /* 1: the inverse mass matrix is shared and re-estimated by the CALLER from the pooled
                                    statistics of all chains at each window end (b2h_welford_pooled_update): the engine
-                                   runs the per-chain dual averaging only and never touches the metric; any metric kind */
+                                   runs the per-chain dual averaging only and never touches the metric; any metric kind.
+                                   The same mode serves a caller that adapts per-chain DENSE matrices itself
+                                   (B2H_IMM_DENSE_PER_CHAIN): it folds the stored draws with b2h_welford_update(full = 1)
+                                   and refactors with b2h_dense_factor_per_chain at each window end                   */
     int32_t step_offset;        /* schedule index of the call's first transition (a warm-up run in several calls)    */
 } b2h_adapt;
 
@@ -252,7 +263,7 @@ int b2h_termination_update(b2h_ctx*, int dtype, void* momentum_ckpts, void* mome
 int b2h_is_iterative_turning(b2h_ctx*, const b2h_metric*, int dtype, const void* momentum_ckpts,
                              const void* momentum_sum_ckpts, const int64_t* idx_min, const int64_t* idx_max,
                              const void* momentum_sum, const void* momentum, uint8_t* out, int64_t C, int64_t d,
-                             int32_t max_num_doublings /* diag-family metrics */);
+                             int32_t max_num_doublings /* diag-family metrics; dense kinds: B2H_ERR_UNSUPPORTED */);
 /* termination._find_storage_indices (termination.py:192-235) */
 int b2h_find_storage_indices(b2h_ctx*, const int64_t* step, int64_t* idx_min, int64_t* idx_max, int64_t n);
 
@@ -285,7 +296,8 @@ int32_t b2h_nuts_plan_group(const b2h_model*, const b2h_metric*, const b2h_cfg*,
 int64_t b2h_hmc_workspace_bytes(const b2h_model*, const b2h_metric*, const b2h_cfg*, int64_t C);
 
 /* ---- stand-alone trajectory builders with caller-supplied tree state (every model; scalar / diagonal metrics: the
- *      reference's tree state carries no velocities, which the dense-metric engine needs -- use b2h_nuts_run) ---- */
+ *      reference's tree state carries no velocities, which the dense-metric engine needs -- use b2h_nuts_run; both
+ *      dense kinds return B2H_ERR_UNSUPPORTED) ---- */
 typedef struct {
     void *q, *p, *g; /* [C x d] */
     void* U;         /* [C]     */
@@ -383,6 +395,19 @@ int b2h_philox_fill(b2h_ctx*, uint64_t seed, uint64_t chain_offset, uint64_t tra
 
 /* Dense apply out[C x d] = in[C x d] . M[d x d] (M symmetric): the mass-matrix / precision mat-vec of all chains */
 int b2h_dense_apply(b2h_ctx*, int dtype, const void* in, const void* M, void* out, int64_t C, int64_t d);
+
+/* Per-chain dense apply out[c] = in[c] . M[c] for c < C: in, out [C x d], M [C x d x d] (chain c's matrix at c * d * d),
+ * the mat-vec of a B2H_IMM_DENSE_PER_CHAIN metric.  tri: 0 M full, 1 M upper-triangular, 2 M lower-triangular (the
+ * codes of b2h_gemm_group.tri; the zero half is never read into a result).  Each element is summed over k in ascending
+ * order, so integer inputs give the exact product.  1 <= d <= B2H_DENSE_PER_CHAIN_MAX_DIM. */
+int b2h_dense_apply_per_chain(b2h_ctx*, int dtype, const void* in, const void* M, void* out, int64_t C, int64_t d,
+                              int32_t tri);
+/* Factors the C matrices imm_in [C x d x d] of a B2H_IMM_DENSE_PER_CHAIN metric: imm = (A + A^T) / 2, then in FP64
+ * whatever the dtype L = chol(imm), sqrt_t = L^-1 (lower) and chol_t = L^T (upper).  info[c] (device int32 [C]) is 0,
+ * or k + 1 when pivot k of chain c is not positive; that chain's imm, sqrt_t and chol_t are then NaN.  imm may alias
+ * imm_in.  1 <= d <= B2H_DENSE_PER_CHAIN_MAX_DIM. */
+int b2h_dense_factor_per_chain(b2h_ctx*, int dtype, const void* imm_in, void* imm, void* sqrt_t, void* chol_t,
+                               int32_t* info, int64_t C, int64_t d);
 
 /* Per-chain mean and unbiased variance (float64 [C x d] each) of draws [T][C][d]: the per-GPU part of R-hat. */
 int b2h_chain_moments(b2h_ctx*, int dtype, const void* draws, int64_t T, int64_t C, int64_t d, double* chain_mean,
