@@ -93,6 +93,7 @@ EXPORTS = [
     "b2h_philox_fill", "b2h_dense_apply", "b2h_dense_apply_per_chain", "b2h_dense_factor_per_chain", "b2h_chain_moments", "b2h_chain_autocov", "b2h_tc_gemm_bf16", "b2h_tc_logistic_residual",
     "b2h_tc_gemm_blocked_bf16", "b2h_gemm", "b2h_nuts_expand", "b2h_nuts_subtree", "b2h_proposal_update",
     "b2h_progressive_sampling", "b2h_select_rows", "b2h_user_model_create", "b2h_user_model_create_ad", "b2h_user_model_create_rev",
+    "b2h_user_model_create_warp",
     "b2h_user_model_set_tape_nodes", "b2h_user_model_tape_needed", "b2h_user_model_destroy",
     "b2h_hmc_accept", "b2h_nuts_plan_group", "b2h_welford_pooled_update", "b2h_welford_pooled_workspace_bytes", "b2h_welford_merge",
     "b2h_tick_timer", "b2h_tick_timer_read",

@@ -201,18 +201,37 @@ class UserModel(Model):
     thread per chain;
     the sampler runs it in split mode (one gradient launch per leapfrog tick).  ``data`` is an optional flat array of
     constants handed to the function in the model's dtype.  ``host_fn(q[d]) -> (U, g)`` is an optional NumPy
-    counterpart (used by the tests as the oracle's model); it is never called by the sampler."""
+    counterpart (used by the tests as the oracle's model); it is never called by the sampler.
+
+    ``warp=True`` declares that the source is written in the warp calling convention
+    (``b2h_user_model_create_warp``): each chain is evaluated by one full warp, and the function takes one more
+    argument, ``const Warp& w``::
+
+        template <typename T>
+        __device__ T potential_and_grad(const T* q, T* g, int d, const T* data, const Warp& w);
+        template <typename S, typename T>                                           // autodiff=True
+        __device__ S log_density(const S* q, int d, const T* data, const Warp& w);
+
+    All 32 lanes call it; the typical loop is ``for (int i = w.lane; i < d; i += w.size)``.  ``w.sum(x)`` (for T and
+    S) returns the sum over the lanes, bit-identical on every lane; every lane must call each ``w.sum`` in the same
+    order, and calling it from lane-divergent code is undefined.  U is lane 0's return value (with autodiff, the
+    gradient is that of lane 0's value), so the other lanes' contributions must reach lane 0 through ``w.sum``.  In
+    the hand-written form each element of g is written by exactly one lane.  With autodiff the warp form is reverse
+    mode at every dim (each lane records its own tape; ``tape_nodes`` counts nodes per lane) and its gradient is
+    deterministic.  It suits wide models: the chain's work is spread over 32 lanes."""
     kind = _lib.MODEL_USER
     FORWARD_MAX_DIM = 64          # autodiff: forward mode up to this dim, reverse mode above
 
     def __init__(self, source, dim, data=None, dtype=torch.float64, device=None, host_fn=None, autodiff=False,
-                 tape_nodes=None):
+                 tape_nodes=None, warp=False):
         super().__init__(dtype, device)
         self.dim = int(dim)
         self.autodiff = bool(autodiff)
-        self.reverse = self.autodiff and self.dim > self.FORWARD_MAX_DIM
+        self.warp = bool(warp)
+        self.reverse = self.autodiff and (self.warp or self.dim > self.FORWARD_MAX_DIM)
         if tape_nodes is not None and not self.reverse:
-            raise ValueError(f"tape_nodes applies to reverse-mode models (autodiff=True, dim > {self.FORWARD_MAX_DIM})")
+            raise ValueError(f"tape_nodes applies to reverse-mode models (autodiff=True, dim > {self.FORWARD_MAX_DIM}, "
+                             "or warp=True)")
         self.tape_nodes = 0
         self.source = str(source)
         self.host_fn = host_fn
@@ -221,7 +240,10 @@ class UserModel(Model):
         lib = _lib.load()
         with torch.cuda.device(self.device):
             handle = C.c_void_p()
-            if self.reverse:
+            if self.warp:
+                _lib.check(lib.b2h_user_model_create_warp(self.source.encode(), C.c_int32(self.dim),
+                                                          C.c_int32(int(self.autodiff)), C.byref(handle)))
+            elif self.reverse:
                 _lib.check(lib.b2h_user_model_create_rev(self.source.encode(), C.c_int32(self.dim), C.byref(handle)))
             elif self.autodiff:
                 _lib.check(lib.b2h_user_model_create_ad(self.source.encode(), C.c_int32(self.dim), C.byref(handle)))
@@ -245,7 +267,8 @@ class UserModel(Model):
         if self.reverse:
             n = self._tape_needed()
             if n > self.tape_nodes:
-                raise _lib.B200HMCError(f"reverse-mode user model: a chain needed {n} tape nodes, the capacity is "
+                per = "a lane of a chain" if self.warp else "a chain"
+                raise _lib.B200HMCError(f"reverse-mode user model: {per} needed {n} tape nodes, the capacity is "
                                         f"{self.tape_nodes} (pass tape_nodes >= {n} to UserModel)")
 
     def struct(self):

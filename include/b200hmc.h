@@ -230,6 +230,29 @@ int b2h_user_model_create_rev(const char* cuda_source, int32_t dim, b2h_user_mod
 /* Sets the tape capacity in nodes per chain, 0 <= nodes <= 2^31 - 1 - dim.  The workspace size depends on it: a
  * workspace sized before the change may be too small afterwards. */
 int b2h_user_model_set_tape_nodes(b2h_user_model* model, int64_t nodes);
+/* The warp form: each chain is evaluated by one full warp, for models wide enough to split over 32 lanes.  The source
+ * defines, with autodiff = 0 (hand-written gradient; dim is ignored),
+ *     template <typename T> __device__ T potential_and_grad(const T* q, T* g, int d, const T* data, const Warp& w);
+ * or, with autodiff = 1 (reverse mode, 1 <= dim <= B2H_USER_REV_MAX_DIM),
+ *     template <typename S, typename T> __device__ S log_density(const S* q, int d, const T* data, const Warp& w);
+ * with the arithmetic and functions of b2h_user_model_create_rev.  The prepended header defines
+ *     struct Warp { int lane; static constexpr int size = 32; X sum(X x) const; };
+ * Contract:
+ *  - all 32 lanes of a chain call the function; the typical loop is for (int i = w.lane; i < d; i += w.size);
+ *  - w.sum(x) (x of type T, or S) returns the sum over the 32 lanes by a fixed-order butterfly, bit-identical on every
+ *    lane.  Every lane must call each w.sum, in the same order: calling it from lane-divergent code is undefined;
+ *  - U is lane 0's return value.  The other lanes' return values are ignored (in reverse mode the gradient is that of
+ *    lane 0's value), so their contributions must reach lane 0 through w.sum;
+ *  - hand-written form: each element of g is written by exactly one lane.
+ * In reverse mode each lane records its own tape; capacities and counts (b2h_user_model_set_tape_nodes,
+ * b2h_user_model_tape_needed) are in nodes per lane, the largest over the lanes.  With N nodes, pitch = 32 C and E as
+ * above, the workspace holds the tape, the node adjoints and each chain's dim input Vars (2E bytes each):
+ *     bytes = 256 + 2 * R(N * pitch * 4) + 2 * R(N * pitch * E) + R(N * pitch * E) + R(C * dim * 2E)
+ * The input adjoints accumulate in the chain's g row, in an order that depends only on the chain's own operations: the
+ * gradient is bit-identical run to run and whatever the chain count or the chain's position.  If any lane of a chain
+ * needs more than N nodes, the chain gets U = +inf and g = 0, as above.  A thread-form source does not compile here
+ * (the log is in b2h_last_error()). */
+int b2h_user_model_create_warp(const char* cuda_source, int32_t dim, int32_t autodiff, b2h_user_model** out);
 /* *needed = the largest node count any chain of a reverse-mode handle needed since the previous read (0 if none was
  * evaluated), then resets it.  Copies on the context's stream and synchronises that stream. */
 int b2h_user_model_tape_needed(b2h_ctx* ctx, b2h_user_model* model, int64_t* needed);
