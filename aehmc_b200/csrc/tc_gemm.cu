@@ -25,6 +25,7 @@
 
 #include <algorithm>
 #include <cstdlib>
+#include <type_traits>
 
 #include "common.cuh"
 #include "launch.h"
@@ -1086,11 +1087,63 @@ tc_logistic_fused16_kernel(const __grid_constant__ CUtensorMap map_x, Fused16Arg
             return 0.6931471805599453f * fmaf(0.5f, pacc.x + pacc.y, lg2_approx(prod));
         };
         float urun = 0.f;
+        // One work item L of a segment: S(L) -> residual pieces in tensor memory, its potential terms added to urun.
+        // BUF = L & 1 is a template constant so that every tensor-memory address is an immediate off lane_addr;
+        // ph = (L >> 1) & 1 is the parity of S(L)'s fill and of the previous release of residual buffer BUF.
+        // On entry ra holds (or is receiving) columns [c0, c0 + 8) of S(L); with has_next the same columns of S(L + 1)
+        // are requested before the second half of this item is processed.  partial is set only for the last data
+        // tile when N is not a multiple of FN; lim = N - (first row of the tile) - c0.
+        auto item = [&](auto bufc, uint32_t ph, const float* yp, bool has_next, bool partial, int lim) {
+            constexpr uint32_t BUF = decltype(bufc)::value;
+            float yv[16];
+            if (!partial) {
+#pragma unroll
+                for (int j = 0; j < 16; j += 4) {
+                    const float4 y4 = __ldg(reinterpret_cast<const float4*>(yp + j));
+                    yv[j] = y4.x; yv[j + 1] = y4.y; yv[j + 2] = y4.z; yv[j + 3] = y4.w;
+                }
+            } else {
+#pragma unroll
+                for (int j = 0; j < 16; ++j) yv[j] = (j < lim) ? __ldg(yp + j) : 0.5f;
+            }
+            // The 16 accumulator columns of this thread are read as two halves so that the tensor-memory read of one
+            // half (TMEM reads run at ~64 B/clk per SM: 32 KB per item) overlaps the arithmetic of the other.
+            uint32_t p0[8], p1[8];
+            float uacc = 0.f;
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");          // ra = columns [c0, c0 + 8) of S(L)
+            tmem_ld8(lane_addr + (uint32_t)c0 + (BUF * FN + 8), rb8);
+            uacc += half_item(ra, yv, p0, p1);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");          // rb8 = columns [c0 + 8, c0 + 16)
+            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&s_empty[BUF])) : "memory");
+            if (has_next) {
+                mbar_wait_backoff(&s_full[BUF ^ 1], ph ^ BUF);
+                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tmem_ld8(lane_addr + (uint32_t)c0 + ((BUF ^ 1) * FN), ra);
+            }
+            uacc += half_item(rb8, yv + 8, p0 + 4, p1 + 4);
+            // rows past the end of the data (s = 0 from the zero-filled X rows, y loaded as 1/2): the residual is 0 by
+            // construction and each such row added log 2 to the potential
+            if (partial) uacc -= 0.6931471805599453f * (float)min(16, max(0, 16 - lim));
+            urun += uacc;
+            // residual pieces -> tensor memory (the second product of item L - 2 must have consumed this buffer)
+            mbar_wait(&r_empty[BUF], ph ^ 1);
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            const uint32_t raddr = lane_addr + (uint32_t)(part * 8) + (H_COL_R + BUF * H_RBUF_COLS);
+            tmem_st8(raddr, p0);
+            tmem_st8(raddr + H_RPIECE_COLS, p1);
+            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&r_full[BUF])) : "memory");
+        };
+        const std::integral_constant<uint32_t, 0> buf0;
+        const std::integral_constant<uint32_t, 1> buf1;
         int segs_done = 0;
-        int m_tile = t_begin / tiles_n, n_tile = t_begin - m_tile * tiles_n;
-        bool first_of_seg = true;
-        for (int t = t_begin, L = 0; t < t_end; ++t, ++L) {
-            if (first_of_seg) {
+        // one pass per segment: the items of one chain tile within this CTA's range
+        for (int t = t_begin, L = 0; t < t_end;) {
+            const int m_tile = t / tiles_n, n_first = t - m_tile * tiles_n;
+            const int cnt = min(t_end - t, tiles_n - n_first);
+            {
                 // beta pieces of this chain tile -> tensor memory (the first products of the previous segment retired)
                 mbar_wait(a_free, (segs_done & 1) ^ 1);
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -1114,59 +1167,34 @@ tc_logistic_fused16_kernel(const __grid_constant__ CUtensorMap map_x, Fused16Arg
                 __syncwarp();
                 if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(a_full)) : "memory");
             }
-            const int n0 = n_tile * FN;
-            const int buf = L & 1;
-            const bool full = n0 + FN <= fa.N;
-            float yv[16];
-            if (full) {
-#pragma unroll
-                for (int j = 0; j < 16; j += 4) {
-                    const float4 y4 = __ldg(reinterpret_cast<const float4*>(fa.y + n0 + c0 + j));
-                    yv[j] = y4.x; yv[j + 1] = y4.y; yv[j + 2] = y4.z; yv[j + 3] = y4.w;
-                }
-            } else {
-#pragma unroll
-                for (int j = 0; j < 16; ++j) yv[j] = (n0 + c0 + j < fa.N) ? __ldg(fa.y + n0 + c0 + j) : 0.5f;
-            }
-            // The 16 accumulator columns of this thread are read as two halves so that the tensor-memory read of one
-            // half (TMEM reads run at ~64 B/clk per SM: 32 KB per item) overlaps the arithmetic of the other; the
-            // first half of the NEXT item is requested before the second half of this one is processed.
-            uint32_t p0[8], p1[8];
-            float uacc = 0.f;
-            if (first_of_seg) {          // nothing was requested ahead (the beta pieces had to be in place first)
-                mbar_wait_backoff(&s_full[buf], (L >> 1) & 1);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                tmem_ld8(lane_addr + (uint32_t)(buf * FN + c0), ra);
-            }
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");          // ra = columns [c0, c0 + 8) of S(L)
-            tmem_ld8(lane_addr + (uint32_t)(buf * FN + c0 + 8), rb8);
-            uacc += half_item(ra, yv, p0, p1);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");          // rb8 = columns [c0 + 8, c0 + 16)
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&s_empty[buf])) : "memory");
-            if (t + 1 < t_end && n_tile + 1 != tiles_n) {      // next item of the same segment
-                const int nbuf = (L + 1) & 1;
-                mbar_wait_backoff(&s_full[nbuf], ((L + 1) >> 1) & 1);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                tmem_ld8(lane_addr + (uint32_t)(nbuf * FN + c0), ra);
-            }
-            uacc += half_item(rb8, yv + 8, p0 + 4, p1 + 4);
-            if (!full) uacc -= 0.6931471805599453f * (float)min(16, max(0, n0 + c0 + 16 - fa.N));
-            urun += uacc;
-            {
-                const int rb = L & 1;
-                mbar_wait(&r_empty[rb], ((L >> 1) & 1) ^ 1);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const uint32_t raddr = lane_addr + H_COL_R + (uint32_t)rb * H_RBUF_COLS + (uint32_t)(part * 8);
-                tmem_st8(raddr, p0);
-                tmem_st8(raddr + H_RPIECE_COLS, p1);
-                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-                asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&r_full[rb])) : "memory");
-            }
+            // nothing was requested ahead for the first item (the beta pieces had to be in place first)
+            mbar_wait_backoff(&s_full[L & 1], (L >> 1) & 1);
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tmem_ld8(lane_addr + (uint32_t)((L & 1) * FN + c0), ra);
 
-            const bool last_of_seg = (t + 1 >= t_end) || (n_tile + 1 == tiles_n);
-            if (last_of_seg) {
+            // steady state: every item but the last of the segment is a full data tile followed by one more item;
+            // pairs start on an even L so that both buffer indices are constants
+            const float* yp = fa.y + n_first * FN + c0;
+            uint32_t ph = (L >> 1) & 1;
+            int k = cnt - 1;
+            if (k > 0 && (L & 1)) { item(buf1, ph, yp, true, false, FN); ph ^= 1; yp += FN; --k; }
+            for (; k >= 2; k -= 2) {
+                item(buf0, ph, yp, true, false, FN);
+                item(buf1, ph, yp + FN, true, false, FN);
+                ph ^= 1;
+                yp += 2 * FN;
+            }
+            if (k) { item(buf0, ph, yp, true, false, FN); yp += FN; }
+
+            // last item of the segment: nothing to request ahead; the last data tile may be partial
+            const int L_last = L + cnt - 1, n_last = n_first + cnt - 1;
+            const bool partial = n_last * FN + FN > fa.N;
+            const int lim = fa.N - n_last * FN - c0;
+            if (L_last & 1) item(buf1, (uint32_t)(L_last >> 1) & 1, yp, false, partial, lim);
+            else item(buf0, (uint32_t)(L_last >> 1) & 1, yp, false, partial, lim);
+
+            {
+                // drain G: this warp's lane quadrant, columns [32 part, 32 part + 32)
                 mbar_wait(g_full, segs_done & 1);
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 uint32_t gq[32];
@@ -1204,8 +1232,8 @@ tc_logistic_fused16_kernel(const __grid_constant__ CUtensorMap map_x, Fused16Arg
                 }
                 urun = 0.f;
             }
-            first_of_seg = last_of_seg;
-            if (++n_tile == tiles_n) { n_tile = 0; ++m_tile; }
+            t += cnt;
+            L += cnt;
         }
     }
 
