@@ -127,6 +127,13 @@ __device__ __forceinline__ float2 fmul2(float2 a, float2 b) {
     asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(rd) : "l"(ra), "l"(rb));
     return *reinterpret_cast<float2*>(&rd);
 }
+// rr + (-float(h)) in one f32 = f16 + f32 instruction (sm_100, FHADD) that reads h, negated, from its half of a packed
+// word: no unpacking to f32 first.  Exact when h = fp16(rr), and +0 when rr is fp16-exact (not -(h - rr), which is -0).
+__device__ __forceinline__ float sub_f16(float rr, __half h) {
+    float d;
+    asm("{\n.reg .b16 n;\nneg.f16 n, %1;\nadd.rn.f32.f16 %0, n, %2;\n}" : "=f"(d) : "h"(__half_as_ushort(h)), "f"(rr));
+    return d;
+}
 __device__ __forceinline__ bool elect_one() {
     uint32_t pred;
     asm volatile(
@@ -1055,7 +1062,7 @@ tc_logistic_fused16_kernel(const __grid_constant__ CUtensorMap map_x, Fused16Arg
         // special functions batched: one ex2 per element, one rcp per PAIR (1/a = b / (a b)), one lg2 per 8 elements
         // (sum of logs = log of the product; every factor is in (1, 2]).
         auto half_item = [&](const uint32_t* r, const float* y, uint32_t* q0, uint32_t* q1) -> float {
-            float2 pacc = make_float2(0.f, 0.f);
+            float2 pacc;
             float2 den2[4], num2[4];
             float pp[4];
             const float2 lscale = make_float2(l2_scale, l2_scale), one2 = make_float2(1.f, 1.f);
@@ -1066,8 +1073,9 @@ tc_logistic_fused16_kernel(const __grid_constant__ CUtensorMap map_x, Fused16Arg
                 const float2 e2 = make_float2(ex2_approx(-fabsf(t2.x)), ex2_approx(-fabsf(t2.y)));
                 den2[h] = fadd2(e2, one2);
                 num2[h] = make_float2(sv2.x >= 0.f ? 1.f : e2.x, sv2.y >= 0.f ? 1.f : e2.y);   // numerator of sigmoid(s)
-                pacc.x += fabsf(t2.x);
-                pacc.y += fabsf(t2.y);
+                // |t| sums per lane, packed (FADD2 takes |.| operands); starting from the first |t| has the bits of 0 + |t|
+                const float2 at2 = make_float2(fabsf(t2.x), fabsf(t2.y));
+                pacc = h == 0 ? at2 : fadd2(pacc, at2);
                 pp[h] = den2[h].x * den2[h].y;
             }
 #pragma unroll
@@ -1076,13 +1084,13 @@ tc_logistic_fused16_kernel(const __grid_constant__ CUtensorMap map_x, Fused16Arg
                 const float2 inv2 = fmul2(make_float2(den2[h].y, den2[h].x), make_float2(rp, rp));
                 const float2 rr = ffma2(num2[h], inv2, make_float2(-y[2 * h], -y[2 * h + 1]));     // sigmoid(s) - y
                 const __half2 hi = __floats2half2_rn(rr.x, rr.y);
-                const float2 hf = __half22float2(hi);
-                const float2 lo2 = fadd2(rr, make_float2(-hf.x, -hf.y));
-                const __half2 lo = __floats2half2_rn(lo2.x, lo2.y);
+                const __half2 lo = __floats2half2_rn(sub_f16(rr.x, __low2half(hi)), sub_f16(rr.y, __high2half(hi)));
                 q0[h] = *reinterpret_cast<const uint32_t*>(&hi);
                 q1[h] = *reinterpret_cast<const uint32_t*>(&lo);
             }
-            const float prod = (pp[0] * pp[1]) * (pp[2] * pp[3]);
+            // (pp0 pp1, pp2 pp3) as one packed product
+            const float2 pq = fmul2(make_float2(pp[0], pp[2]), make_float2(pp[1], pp[3]));
+            const float prod = pq.x * pq.y;
             // sum of 1/2 |s| + log(1 + exp(-|s|)):  |s| = |t| ln 2
             return 0.6931471805599453f * fmaf(0.5f, pacc.x + pacc.y, lg2_approx(prod));
         };

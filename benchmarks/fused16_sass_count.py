@@ -1,20 +1,30 @@
 """Instruction count of the steady-state item path of the fp16 x 2 fused logistic gradient's epilogue, per instantiation
-(KB = 1: dim <= 64, KB = 2: dim <= 128), from `cuobjdump -sass` of the built library, split into the floating-point
-arithmetic of half_item and everything else.
+(KB = 1: dim <= 64, KB = 2: dim <= 128), from `cuobjdump -sass` of the built library (or of a cubin), split into the
+floating-point arithmetic of half_item and everything else.  --cu compiles one source file to a cubin with the
+Makefile's flags in a temporary directory and counts that: no library build or link is needed.
 
 By default the path is the innermost loop of the kernel that holds a full work item (16 MUFU.EX2 per item), and the
 count is per item (the loop runs two items per trip).  --ranges counts explicit half-open address ranges instead (for
 builds without that loop), e.g. --ranges 2:0x15b0-0x1660,0x1ab0-0x29f0 --ranges 1:...; a static count of what lies in
 the ranges.
-    python benchmarks/fused16_sass_count.py [--lib aehmc_b200/lib/libb200hmc.so] [--ranges KB:A-B,...]"""
-import argparse, collections, os, re, subprocess
+    python benchmarks/fused16_sass_count.py [--lib aehmc_b200/lib/libb200hmc.so | --cu aehmc_b200/csrc/tc_gemm.cu]
+                                            [--ranges KB:A-B,...]"""
+import argparse, collections, os, re, subprocess, tempfile
 
-ARITH = {"MUFU", "FMUL", "FADD", "FFMA", "FMUL2", "FADD2", "FFMA2", "FSETP", "FSEL", "F2FP", "HADD2"}
+ARITH = {"MUFU", "FMUL", "FADD", "FFMA", "FMUL2", "FADD2", "FFMA2", "FSETP", "FSEL", "F2FP", "HADD2", "FHADD", "FHFMA"}
 KERNEL = "_ZN3b2h2tc26tc_logistic_fused16_kernelILi{}EEEv14CUtensorMap_stNS0_11Fused16ArgsE"
+CUDA = os.environ.get("CUDA_HOME", "/usr/local/cuda")
+
+
+def cubin(src, out_dir):
+    out = os.path.join(out_dir, os.path.splitext(os.path.basename(src))[0] + ".cubin")
+    subprocess.run([os.path.join(CUDA, "bin", "nvcc"), "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17",
+                    "-lineinfo", "--expt-relaxed-constexpr", "-cubin", src, "-o", out], check=True)
+    return out
 
 
 def sass(lib, kb):
-    cuobjdump = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
+    cuobjdump = os.path.join(CUDA, "bin", "cuobjdump")
     txt = subprocess.run([cuobjdump, "-sass", "-fun", KERNEL.format(kb), lib], check=True, capture_output=True,
                          text=True).stdout
     ins = [(int(m.group(1), 16), m.group(2)) for m in re.finditer(r"/\*([0-9a-f]{4,})\*/\s+([^;]*?)\s*;", txt)]
@@ -45,15 +55,20 @@ def steady_loop(ins):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--lib", default="aehmc_b200/lib/libb200hmc.so")
+    src = ap.add_mutually_exclusive_group()
+    src.add_argument("--lib", default="aehmc_b200/lib/libb200hmc.so", help="library or cubin to disassemble")
+    src.add_argument("--cu", help="source file to compile to a cubin and disassemble")
     ap.add_argument("--ranges", action="append", default=[], help="KB:A-B,C-D (half-open, hex)")
     a = ap.parse_args()
     given = {}
     for spec in a.ranges:
         kb, rs = spec.split(":")
         given[int(kb)] = [tuple(int(x, 16) for x in r.split("-")) for r in rs.split(",")]
+    with tempfile.TemporaryDirectory() as tmp:
+        lib = cubin(a.cu, tmp) if a.cu else a.lib
+        ins_by_kb = {kb: sass(lib, kb) for kb in (1, 2)}
     for kb in (1, 2):
-        ins = sass(a.lib, kb)
+        ins = ins_by_kb[kb]
         if kb in given:
             ranges, items, how = given[kb], 1, "given ranges"
         else:
